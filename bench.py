@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload cfg3|cfg4|cfg5|cfg1like] [--sites K] [--chains C] [--siter I]
                     [--damp auto|schedule] [--data sim|synth] [--max-treedepth T] [--rhat-max R]
+                    [--dump-outputs DIR]
 
     python bench.py --workload cfg5 --sites 148 --siter 100 --max-treedepth 6 --rhat-max 0 --no-cpu-baseline
         BASELINE.json configs[4] (K=256, n_k=200 000, D=199, 32 chains), bounded: one wave of sites, 100
@@ -324,6 +325,25 @@ def run_reference(args, model, K, n_k, D, chains, siter):
     print(json.dumps(line))
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, m, m_phi, cov_phi):
+    """What the last timed EP iteration computed, as float64 .npy files in `out_dir`, so that two builds run
+    with the same arguments can be compared output for output: the global approximation Master.run returned
+    (m_phi, cov_phi), its natural parameters (Q, r) and the site natural parameters (site_Qi [d, d, n],
+    site_ri [d, n]) of the sites in site_index -- all K sites, or a fixed seeded sample of them when all would
+    exceed DUMP_BYTES in all."""
+    d, K = m.dphi, m.K
+    per_site = 8 * (d * d + d + 1)
+    n = min(K, (DUMP_BYTES - 16 * (d * d + d) - 7 * 128) // per_site)      # (128: an .npy header)
+    idx = np.arange(K) if n == K else np.sort(np.random.RandomState(0).choice(K, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (('m_phi', m_phi), ('cov_phi', cov_phi), ('Q', m.Q), ('r', m.r),
+                    ('site_Qi', m.Qi[:, :, idx]), ('site_ri', m.ri[:, idx]), ('site_index', idx)):
+        np.save(os.path.join(out_dir, name + '.npy'), np.asarray(a, dtype=np.float64))
+
+
 def run_ours(args, model, K, n_k, D, chains, siter):
     import torch
     import torch.distributed as dist
@@ -427,6 +447,10 @@ def run_ours(args, model, K, n_k, D, chains, siter):
     clocks = ClockSampler(local_rank) if rank == 0 else None
     done, ms_dev, ms_wall, launches = timed_run(args.steps)
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs:
+        m.sync_host()                  # (every rank: the site arrays are gathered over the ranks)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, m, hist['m'][-1], hist['S'][-1])
     samp_s = float(np.sum(hist['stime'][i_timed:]))
     evals = torch.tensor([float(m.n_leapfrog_total)], dtype=torch.float64, device='cuda')
     if world > 1:
@@ -565,7 +589,13 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--max-treedepth', type=int, default=None,
                     help="NUTS control (Stan's default 10); bounds the step time of --workload cfg5, stated in config")
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed EP iteration computed to DIR/<name>.npy (float64, <= 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs needs --impl ours (the reference arm times sampling only)')
     model, K, n_k, D, chains, siter = WORKLOADS[args.workload]
     K = args.sites or K
     chains = args.chains or chains

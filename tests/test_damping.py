@@ -79,54 +79,48 @@ def test_reference_schedule_diverges_selection_converges_oracle():
     assert kl_full[0] < 0.5 * kl_ref[0] and kl_full.max() < 0.6 * kl_ref[0]
 
 
-def test_master_selection_matches_oracle_cpu():
+def test_master_selection_matches_oracle_cpu(monkeypatch):
     """Host logic of df_select='snr' (fake device context) == oracle replay of the same rule."""
     sys.path.insert(0, TESTS)
     import epstan.method as method
     import fake_backend
-    old = method.Master._context_factory
-    method.Master._context_factory = staticmethod(lambda dev, stream: fake_backend.OracleContext(dev, stream))
-    try:
-        sc = _scenario(K=12, d=6, chains=4, it=60, niter=6, seed=11, df0=orc.default_df0(12))
-        m = _master(method, sc, df_select='snr')
-        info, (ms, Ss) = m.run(sc['niter'], verbose=False, seed=sc['seed'])
-        oinfo, oms, oSs, st, _ = _oracle_run(sc, df_select='snr')
-        assert info == oinfo == 0
-        assert relerr(ms, oms) < 1e-10 and relerr(Ss, oSs) < 1e-10
-        assert len(m.history['df']) == sc['niter'] and len(m.history['snr']) == sc['niter']
-        assert all(m.df_min <= v <= 0.5 for v in m.history['df'])
-        # bad option values
-        with pytest.raises(ValueError):
-            _master(method, sc, df_select='best')
-    finally:
-        method.Master._context_factory = old
+    monkeypatch.setattr(method.Master, '_context_factory',
+                        staticmethod(lambda dev, stream: fake_backend.OracleContext(dev, stream)))
+    sc = _scenario(K=12, d=6, chains=4, it=60, niter=6, seed=11, df0=orc.default_df0(12))
+    m = _master(method, sc, df_select='snr')
+    info, (ms, Ss) = m.run(sc['niter'], verbose=False, seed=sc['seed'])
+    oinfo, oms, oSs, st, _ = _oracle_run(sc, df_select='snr')
+    assert info == oinfo == 0
+    assert relerr(ms, oms) < 1e-10 and relerr(Ss, oSs) < 1e-10
+    assert len(m.history['df']) == sc['niter'] and len(m.history['snr']) == sc['niter']
+    assert all(m.df_min <= v <= 0.5 for v in m.history['df'])
+    # bad option values
+    with pytest.raises(ValueError):
+        _master(method, sc, df_select='best')
 
 
-def test_host_state_is_not_rewound_cpu():
+def test_host_state_is_not_rewound_cpu(monkeypatch):
     """ADVICE r1: a keep_on_device run leaves the host mirrors stale; the next host-state run must
     refresh them instead of uploading the stale copies over the newer device state."""
     sys.path.insert(0, TESTS)
     import epstan.method as method
     import fake_backend
-    old = method.Master._context_factory
-    method.Master._context_factory = staticmethod(lambda dev, stream: fake_backend.OracleContext(dev, stream))
-    try:
-        sc = _scenario(K=6, d=5, chains=4, it=60, niter=3, seed=5, df0=0.3)
-        a = _master(method, sc)
-        b = _master(method, sc)
-        a.run(2, verbose=False, seed=1)
-        a.run(2, verbose=False, seed=2)
-        ia, (ma, Sa) = a.run(2, verbose=False, seed=3)
-        b.run(2, verbose=False, seed=1)
-        b.keep_on_device = True
-        b.run(2, verbose=False, seed=2)
-        assert b._host_stale
-        b.keep_on_device = False
-        ib, (mb, Sb) = b.run(2, verbose=False, seed=3)
-        assert ia == ib == 0 and not b._host_stale
-        assert relerr(mb, ma) < 1e-12 and relerr(Sb, Sa) < 1e-12 and relerr(b.Qi, a.Qi) < 1e-12
-    finally:
-        method.Master._context_factory = old
+    monkeypatch.setattr(method.Master, '_context_factory',
+                        staticmethod(lambda dev, stream: fake_backend.OracleContext(dev, stream)))
+    sc = _scenario(K=6, d=5, chains=4, it=60, niter=3, seed=5, df0=0.3)
+    a = _master(method, sc)
+    b = _master(method, sc)
+    a.run(2, verbose=False, seed=1)
+    a.run(2, verbose=False, seed=2)
+    ia, (ma, Sa) = a.run(2, verbose=False, seed=3)
+    b.run(2, verbose=False, seed=1)
+    b.keep_on_device = True
+    b.run(2, verbose=False, seed=2)
+    assert b._host_stale
+    b.keep_on_device = False
+    ib, (mb, Sb) = b.run(2, verbose=False, seed=3)
+    assert ia == ib == 0 and not b._host_stale
+    assert relerr(mb, ma) < 1e-12 and relerr(Sb, Sa) < 1e-12 and relerr(b.Qi, a.Qi) < 1e-12
 
 
 # ------------------------------------------------------------------------------------- GPU
