@@ -58,6 +58,7 @@ static void free_state(epg_ctx* c) {
     if (c->chol) cudaFree(c->chol); c->chol = nullptr;
     if (c->site_ok) cudaFree(c->site_ok); c->site_ok = nullptr;
     if (c->flags) cudaFree(c->flags); c->flags = nullptr;
+    c->sums_valid = false;         // q_prev / snr_buf describe the old state (and may be too small for the new one)
 }
 
 extern void epg_sites_free(epg_ctx* c);
@@ -127,6 +128,7 @@ int epg_init_state(epg_ctx* c, int K, int d) {
     }
     EPG_CHECK(c, cudaMalloc((void**)&c->chol, sizeof(double) * (size_t)d * (d + 1) / 2));
     EPG_CHECK(c, cudaMalloc((void**)&c->site_ok, sizeof(int) * (size_t)K));
+    EPG_CHECK(c, cudaMemsetAsync(c->site_ok, 0, sizeof(int) * (size_t)K, c->stream));   // no site has a result yet
     EPG_CHECK(c, cudaMalloc((void**)&c->flags, sizeof(int) * 8));
     EPG_CHECK(c, cudaMemsetAsync(c->flags, 0, sizeof(int) * 8, c->stream));
     if (ensure_hflags(c, (size_t)K + 8)) return -1;

@@ -43,7 +43,9 @@ struct epg_ctx {
     // global (Q, r) at the time of the last epg_delta_sums: base of epg_update_from_sums
     double* q_prev = nullptr;
     size_t q_prev_bytes = 0;
-    bool q_prev_valid = false;
+    // q_prev, snr_buf and EPG_DSUM were filled by epg_delta_sums(_ex) for the current state (K, d);
+    // cleared by epg_init_state, required by epg_update_from_sums and epg_delta_snr
+    bool sums_valid = false;
 
     // scratch of the damping-selection statistics (epg_snr.cu)
     double* snr_buf = nullptr;

@@ -244,6 +244,7 @@ int epg_delta_sums_ex(epg_ctx* c, int with_norms, const double* slots, int n_slo
     const int d = c->d, K = c->K;
     const size_t dd = (size_t)d * d;
     const SnrPlan p = snr_plan(K, d);
+    c->sums_valid = false;                                        // (until this call has completed)
     EPG_CHECK(c, epg_reserve((void**)&c->snr_buf, &c->snr_bytes, sizeof(double) * p.total));
     double* buf = c->snr_buf;
     int* flag = reinterpret_cast<int*>(buf + p.o_flag);
@@ -261,7 +262,6 @@ int epg_delta_sums_ex(epg_ctx* c, int with_norms, const double* slots, int n_slo
     EPG_CHECK(c, epg_reserve((void**)&c->q_prev, &c->q_prev_bytes, sizeof(double) * (dd + d)));
     EPG_CHECK(c, cudaMemcpyAsync(c->q_prev, c->arr[EPG_Q], sizeof(double) * dd, cudaMemcpyDeviceToDevice, c->stream));
     EPG_CHECK(c, cudaMemcpyAsync(c->q_prev + dd, c->arr[EPG_R], sizeof(double) * d, cudaMemcpyDeviceToDevice, c->stream));
-    c->q_prev_valid = true;
     // DSUM = [sum dQi | sum dri | sum |delta_k|^2 | n_ok | slots]   (failed sites hold zero deltas: method.py:460-465)
     double* dsum = c->arr[EPG_DSUM];
     {
@@ -282,11 +282,12 @@ int epg_delta_sums_ex(epg_ctx* c, int with_norms, const double* slots, int n_slo
     SNR_LAUNCH_CHECK(c);
     k_sum_norms<<<1, 256, 0, c->stream>>>(buf + p.o_norm, c->site_ok, K, dsum + dd + d);
     SNR_LAUNCH_CHECK(c);
+    c->sums_valid = true;
     return 0;
 }
 
 int epg_delta_snr(epg_ctx* c, double* stats_out) {
-    if (!c->arr[EPG_Q] || !c->snr_buf) return epg_fail_msg(c, "epg_delta_snr: call epg_delta_sums first");
+    if (!c->arr[EPG_Q] || !c->sums_valid) return epg_fail_msg(c, "epg_delta_snr: call epg_delta_sums(_ex) first");
     const int d = c->d, K = c->K;
     const size_t dd = (size_t)d * d;
     const SnrPlan p = snr_plan(K, d);
@@ -339,7 +340,7 @@ int epg_mix_phi_sums(epg_ctx* c, int n, double* sums_out) {
 }
 
 int epg_update_from_sums(epg_ctx* c, double df) {
-    if (!c->arr[EPG_Q] || !c->q_prev_valid) return epg_fail_msg(c, "epg_update_from_sums: call epg_delta_sums(_ex) first");
+    if (!c->arr[EPG_Q] || !c->sums_valid) return epg_fail_msg(c, "epg_update_from_sums: call epg_delta_sums(_ex) first");
     const int d = c->d, E = d * d + d;
     k_partial_from_sums<<<(E + 255) / 256, 256, 0, c->stream>>>(c->q_prev, c->arr[EPG_Q0], c->arr[EPG_R0],
                                                                c->arr[EPG_DSUM], c->arr[EPG_PARTIAL], df, d);

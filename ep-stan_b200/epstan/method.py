@@ -741,7 +741,11 @@ class Master(object):
         if j_all >= BIG:
             return 2, df_first, 0
         if j_all != j:
-            df = df_first * self.df_decay ** j_all
+            # the damping the ladder reaches at position j_all, bit for bit: the ranks whose own ladder stopped
+            # there multiplied by df_decay j_all times (df_first * df_decay ** j_all rounds differently)
+            df = df_first
+            for _ in range(j_all):
+                df *= self.df_decay
             if attempt(df) != 1:
                 raise RuntimeError("damping consensus: a smaller damping factor failed where a larger one passed")
         return 0, df, j_all + 1

@@ -96,7 +96,13 @@ int64_t epg_array_count(epg_ctx* ctx, int array, int k0, int k1);
 
 /* ---- cavity: Worker.cavity, method.py:267-302 (batched over sites) ----
  * proposal==0 uses (Qi,ri), 1 uses (Qi2,ri2).  Writes EPG_CAVQ / EPG_CAVM for
- * sites whose cavity is pos.def.; posdef_out[k1-k0] (may be NULL); *all_ok. */
+ * sites whose cavity is pos.def.; posdef_out[k1-k0] (may be NULL); *all_ok.
+ *
+ * Site flags: the context keeps ONE per-site flag vector, written by the last
+ * per-site call that covered the site -- epg_moments (moment estimate ok),
+ * epg_fail_sites (cleared), epg_cavity (cavity pos.def.) and epg_force_pd
+ * (site forced).  epg_delta_sums(_ex) counts it as n_ok and skips the Fisher
+ * norms of flagged-off sites, so call it right after epg_moments/epg_fail_sites. */
 int epg_cavity(epg_ctx* ctx, int k0, int k1, int proposal, int32_t* posdef_out, int* all_ok);
 
 /* ---- moment matching: Worker.tilted second half, method.py:408-468 ----
@@ -151,7 +157,9 @@ int epg_delta_snr(epg_ctx* ctx, double* stats_out);
  * epg_update_from_sums: with EPG_DSUM all-reduced, sets EPG_PARTIAL so that the following
  *   epg_update_finish yields the proposal Q = Q_prev + df * sum_k dQi, r = r_prev + df * sum_k dri --
  *   identical on every rank, so damping retries need no further exchange of matrices
- *   (epg_update_partial(df) still forms the local Qi2 = Qi + df dQi for the proposal cavities). */
+ *   (epg_update_partial(df) still forms the local Qi2 = Qi + df dQi for the proposal cavities).
+ * epg_delta_snr and epg_update_from_sums fail (return < 0) unless epg_delta_sums(_ex) has run since the
+ *   last epg_init_state: the snapshot and the sums belong to one state. */
 int epg_delta_sums_ex(epg_ctx* ctx, int with_norms, const double* slots, int n_slots);
 
 /* ---- Master.mix_phi, method.py:1250-1301: pool the last tilted draws of phi over the sites ----

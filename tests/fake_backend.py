@@ -6,6 +6,7 @@ container without a GPU.  Lives under tests/: the product never imports it."""
 import numpy as np
 import torch
 
+from epstan._lib import EpgError
 from oracle import ep_linalg as orc
 
 (Q, R, Q0, R0, QI, RI, QI2, RI2, DQI, DRI, CAVQ, CAVM, S, M, PARTIAL, TMEAN, DSUM) = range(17)
@@ -36,7 +37,7 @@ class OracleContext(object):
         self.a[DSUM] = np.zeros(d * d + d + 2 + XCHG_SLOTS)
         self._qprev = None
         self._dsum_t = torch.from_numpy(self.a[DSUM])
-        self._ok = np.ones(K, dtype=bool)
+        self._ok = np.zeros(K, dtype=bool)    # (epg_init_state clears the site flags)
         self.draws = None
         self.U = None
 
@@ -80,9 +81,16 @@ class OracleContext(object):
         self.a[DSUM][d * d + d] = S2
         self.a[DSUM][d * d + d + 1] = self._ok.sum()
 
+    def _sums(self, what):
+        if self._qprev is None:
+            raise EpgError(what + ": call epg_delta_sums(_ex) first")
+        return self._qprev
+
     def delta_snr(self):
+        # (the Fisher metric of the (Q, r) that delta_sums snapshotted, as epg_delta_snr)
         d = self.d
-        T2 = orc.fisher_norm2(self.a[Q], self.a[R], self.a[DSUM][:d * d].reshape(d, d, order='F'),
+        Qp, rp = self._sums('epg_delta_snr')
+        T2 = orc.fisher_norm2(Qp, rp, self.a[DSUM][:d * d].reshape(d, d, order='F'),
                               self.a[DSUM][d * d:d * d + d])
         return T2, float(self.a[DSUM][d * d + d]), int(round(self.a[DSUM][d * d + d + 1]))
 
@@ -105,7 +113,7 @@ class OracleContext(object):
 
     def update_from_sums(self, df):
         d = self.d
-        Qp, rp = self._qprev
+        Qp, rp = self._sums('epg_update_from_sums')
         self.a[PARTIAL][:d * d] = ((Qp - self.a[Q0]) + df * self.a[DSUM][:d * d].reshape(d, d, order='F')).ravel(order='F')
         self.a[PARTIAL][d * d:d * d + d] = (rp - self.a[R0]) + df * self.a[DSUM][d * d:d * d + d]
 
@@ -124,6 +132,7 @@ class OracleContext(object):
             flags[k - k0] = ok
             self.a[CAVQ][:, :, k] = P
             self.a[CAVM][:, k] = mu
+        self._ok[k0:k1] = flags             # epg_cavity owns the site flags too (include/epgpu.h)
         return flags, bool(flags.all())
 
     def set_draws(self, draws, n, k0=0, k1=None):
@@ -192,6 +201,7 @@ class OracleContext(object):
             if lam[k] < thr:
                 self.a[QI][np.arange(self.d), np.arange(self.d), k] += min_eig - lam[k]
                 forced[k] = True
+        self._ok[:] = forced                # (so does epg_force_pd)
         return forced, lam
 
     def set_option(self, name, value):
