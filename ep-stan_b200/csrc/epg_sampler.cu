@@ -84,6 +84,7 @@ struct epg_site_data {
     size_t out_bytes = 0;
     double* ld_buf = nullptr;           // logdensity staging
     size_t ld_bytes = 0;
+    int32_t plan[EPG_PLAN_FIELDS] = {}; // launch plan of the last epg_tilted_sample / epg_logdensity (epg_last_plan)
 };
 
 void epg_sites_free(epg_ctx* c) {
@@ -1664,11 +1665,14 @@ k_nuts_pp(const SamplerArgs a, const __grid_constant__ CUtensorMap tmap, int n_s
     tc::teardown(tmem_base);
 }
 
-// log-density / gradient at caller-supplied points (parity tests)
-template <int CP>
-__global__ void __launch_bounds__(tc::NTHREADS, 1) k_logdensity(const SamplerArgs a, const __grid_constant__ CUtensorMap tmap,
-                                                           int nq, double* lp_out, double* grad_out) {
+// log-density / gradient at caller-supplied points (parity tests): the likelihood pass of k_nuts<CP, TCM>, run
+// `ticks` times, then the gradient finish of its chain phase (the same ChainCtxT)
+template <int CP, int TCM>
+__global__ void __launch_bounds__(TCM ? tc::NTHREADS : NTHR, 1)
+k_logdensity(const SamplerArgs a, const __grid_constant__ CUtensorMap tmap, int nq, int ticks, double* lp_out,
+             double* grad_out) {
     extern __shared__ __align__(1024) unsigned char smem[];
+    constexpr bool USE_TC = TCM == 1, USE_TCW = TCM == 2;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int k_local = a.k0;
     const int d = a.d, D = a.D, S = a.S;
@@ -1682,12 +1686,8 @@ __global__ void __launch_bounds__(tc::NTHREADS, 1) k_logdensity(const SamplerArg
     float* om = a.omega_smem ? reinterpret_cast<float*>(smem + a.off_omega)
                              : a.omega + (size_t)k_local * (d * d + d);
     float* muf = om + d * d;
-    const double* cq = a.cavQ + (size_t)k_local * d * d;
-    if (worker) {
-        for (int e = tid; e < d * d; e += NTHR) om[e] = (float)cq[e];
-        for (int i = tid; i < d; i += NTHR) muf[i] = (float)a.cavm[(size_t)k_local * d + i];
-    }
-    if (a.resident && !a.use_tc) {
+    if (worker) load_cavity(a, k_local, om, tid, NTHR);
+    if (TCM == 0 && a.resident) {
         const float4* src = reinterpret_cast<const float4*>(a.X + (size_t)row_begin * S);
         float4* dst = reinterpret_cast<float4*>(smem);
         for (int e = tid; e < n_rows * (S >> 2); e += NTHR) dst[e] = src[e];
@@ -1696,10 +1696,11 @@ __global__ void __launch_bounds__(tc::NTHREADS, 1) k_logdensity(const SamplerArg
     uint32_t tmem_base = 0;
     tc::State tcst;
     tcw::State tcwst;
-    if (a.use_tc == 1) {
+    if constexpr (USE_TC) {
         tcst.set_stages(a.tc_nst);
         tmem_base = tc::setup(tcb, a.tc_nst);
-    } else if (a.use_tc == 2) {
+    }
+    if constexpr (USE_TCW) {
         tcwst.nst = (uint32_t)a.tc_nst;
         tmem_base = tcw::setup(tcb);
     }
@@ -1711,27 +1712,24 @@ __global__ void __launch_bounds__(tc::NTHREADS, 1) k_logdensity(const SamplerArg
         }
     __threadfence_block();
     __syncthreads();
-    if (a.use_tc == 2) {
-        // (twice: exercises the pipeline state carried across ticks)
-        likelihood_pass_tcw(a, smem, tcb, tmem_base, &tmap, tcwst, k_local, nq, row_begin, n_rows, lp_lik, om, muf);
-        likelihood_pass_tcw(a, smem, tcb, tmem_base, &tmap, tcwst, k_local, nq, row_begin, n_rows, lp_lik, om, muf);
-    } else if (a.use_tc) {
-        likelihood_pass_tc(a, smem, tcb, tmem_base, &tmap, tcst, k_local, nq, row_begin, n_rows, lp_lik, om, muf);
-        // second evaluation: exercises the pipeline state carried across ticks
-        likelihood_pass_tc(a, smem, tcb, tmem_base, &tmap, tcst, k_local, nq, row_begin, n_rows, lp_lik, om, muf);
-    } else {
-        likelihood_pass<CP>(a, smem, k_local, k_local, nq, J, row_begin, n_rows, grows, lp_lik, om, muf);
+    // (ticks > 1: the pipeline state of the tensor-core passes carries over from one pass to the next, as it
+    //  does between the sampler's gradient evaluations)
+    for (int t = 0; t < ticks; ++t) {
+        if constexpr (USE_TC) likelihood_pass_tc(a, smem, tcb, tmem_base, &tmap, tcst, k_local, nq, row_begin, n_rows, lp_lik, om, muf);
+        else if constexpr (USE_TCW) likelihood_pass_tcw(a, smem, tcb, tmem_base, &tmap, tcwst, k_local, nq, row_begin, n_rows, lp_lik, om, muf);
+        else likelihood_pass<CP>(a, smem, k_local, k_local, nq, J, row_begin, n_rows, grows, lp_lik, om, muf);
+        __syncthreads();
     }
     for (int c = warp; worker && c < nq; c += NWARP) {
-        const ChainCtxT<false> x = make_chain_ctx<false>(a, SiteView{smem, k_local}, c, p, d, J, D, lane,
-                                                         make_uint2(0u, 0u), om, muf, nullptr);
+        const ChainCtxT<USE_TC> x = make_chain_ctx<USE_TC>(a, SiteView{smem, k_local}, c, p, d, J, D, lane,
+                                                           make_uint2(0u, 0u), om, muf, nullptr);
         const double V = finish_gradient(x, lp_lik[c]);
         const float* g = x.v(V_G);
         if (lane == 0) lp_out[c] = -V;
         for (int i = lane; i < p; i += 32) grad_out[(size_t)c * p + i] = -(double)g[i];
     }
-    if (a.use_tc == 1) tc::teardown(tmem_base);
-    if (a.use_tc == 2) tcw::teardown(tmem_base);
+    if constexpr (USE_TC) tc::teardown(tmem_base);
+    if constexpr (USE_TCW) tcw::teardown(tmem_base);
 }
 
 __global__ void k_set_q(float* chain_mem, int chain0, int P, int p, int nq, const double* q) {
@@ -2130,6 +2128,14 @@ static int fill_args(epg_ctx* c, SamplerArgs& a, int C, int CP, int n_sites = 1,
     return 0;
 }
 
+// what epg_last_plan reports (field order: include/epgpu.h)
+static void record_plan(epg_site_data* s, const SamplerArgs& a, int kernel, int CP) {
+    const int chain_pad = a.use_tc == 2 ? tcw::NCH : (a.use_tc ? (a.C <= 4 ? 4 : (a.C <= 8 ? 8 : 16)) : CP);
+    const int32_t v[EPG_PLAN_FIELDS] = {kernel, a.use_tc, chain_pad, a.use_tc ? a.tc_nst : 0, a.resident, a.R,
+                                        a.slices, a.NC, a.hot_nvec, a.hot_levels, a.omega_smem, (int32_t)a.smem_total};
+    memcpy(s->plan, v, sizeof(v));
+}
+
 int epg_reserve_draws(epg_ctx* c, int n);
 
 int epg_tilted_sample(epg_ctx* c, int k0, int k1, const uint32_t* seeds, const epg_sampler_opts* o,
@@ -2208,6 +2214,7 @@ int epg_tilted_sample(epg_ctx* c, int k0, int k1, const uint32_t* seeds, const e
     else if (CP == 4) LAUNCH_NUTS(4, 0) else if (CP == 8) LAUNCH_NUTS(8, 0)
     else if (CP == 16) LAUNCH_NUTS(16, 0) else LAUNCH_NUTS(32, 0)
     c->launches++;
+    record_plan(s, a, a.pp ? 2 : 1, CP);
     EPG_CHECK(c, cudaGetLastError());
     EPG_CHECK(c, cudaEventRecord(e1, c->stream));
     EPG_CHECK(c, cudaEventSynchronize(e1));
@@ -2305,31 +2312,62 @@ int epg_reinit_sites(epg_ctx* c, int n, const int32_t* sites) {
     return 0;
 }
 
-int epg_logdensity(epg_ctx* c, int k, int nq, const double* q, double* lp_out, double* grad_out) {
-    if (!c->sites || k < 0 || k >= c->K || nq < 1) return epg_fail_msg(c, "epg_logdensity: bad args");
+int epg_logdensity(epg_ctx* c, int k, int nq, const double* q, double* lp_out, double* grad_out, int chains,
+                   int ticks) {
+    if (!c->sites || k < 0 || k >= c->K || nq < 1 || chains > 32 || ticks < 1)
+        return epg_fail_msg(c, "epg_logdensity: bad args");
     epg_site_data* s = c->sites;
     const int p = s->h_p[k];
-    const int C = (s->tc_ok && s->use_tc && s->nkc == 1) ? tc::NCH : 32, CP = 32;
     SamplerArgs a;
+    int C = chains;
+    if (C <= 0) {
+        // default: the most chains (<= 16) at which the sampler keeps the single-box tensor-core pass when that
+        // pass may serve the sites; otherwise 32 (the wide tensor-core pass where it applies, else SIMT)
+        C = 32;
+        if (s->tc_ok && s->use_tc && s->nkc == 1)
+            for (int n = tc::NCH; n >= 1; --n) {
+                memset(&a, 0, sizeof(a));
+                if (fill_args(c, a, n, pad_chains(n), 1, true) == 0 && a.use_tc == 1) { C = n; break; }
+            }
+    }
+    const int CP = pad_chains(C);
     memset(&a, 0, sizeof(a));
-    if (int rc = fill_args(c, a, C, CP)) return rc;
+    // the plan of epg_tilted_sample for C chains on one site
+    if (int rc = fill_args(c, a, C, CP, 1, true)) return rc;
     s->last_C = 0;                                   // chain memory was repurposed
     a.k0 = k;
     const size_t need = sizeof(double) * ((size_t)C * p * 2 + C);
     EPG_CHECK(c, epg_reserve((void**)&s->ld_buf, &s->ld_bytes, need));
     double* dq = s->ld_buf; double* dlp = dq + (size_t)C * p; double* dg = dlp + C;
-    EPG_CHECK(c, set_smem_attr(k_logdensity<32>, a.smem_total));
+#define LAUNCH_LD(CPV, TC)                                                                              \
+    {                                                                                                   \
+        EPG_CHECK(c, set_smem_attr(k_logdensity<CPV, TC>, a.smem_total));                              \
+        k_logdensity<CPV, TC><<<1, TC ? tc::NTHREADS : NTHR, a.smem_total, c->stream>>>(a, s->tmap, nb, ticks, dlp, dg); \
+    }
+    record_plan(s, a, 3, CP);
     for (int q0 = 0; q0 < nq; q0 += C) {
         const int nb = std::min(C, nq - q0);
         EPG_CHECK(c, cudaMemcpyAsync(dq, q + (size_t)q0 * p, sizeof(double) * (size_t)nb * p, cudaMemcpyHostToDevice, c->stream));
         k_set_q<<<(nb * p + 255) / 256, 256, 0, c->stream>>>(s->chain_mem, k * C, s->Pmax, p, nb, dq);
-        k_logdensity<32><<<1, a.use_tc ? tc::NTHREADS : NTHR, a.smem_total, c->stream>>>(a, s->tmap, nb, dlp, dg);
+        // the six instances k_nuts is launched as (epg_tilted_sample)
+        if (a.use_tc == 2) LAUNCH_LD(32, 2)
+        else if (a.use_tc) LAUNCH_LD(32, 1)
+        else if (CP == 4) LAUNCH_LD(4, 0) else if (CP == 8) LAUNCH_LD(8, 0)
+        else if (CP == 16) LAUNCH_LD(16, 0) else LAUNCH_LD(32, 0)
         c->launches += 2;
         EPG_CHECK(c, cudaGetLastError());
         EPG_CHECK(c, cudaMemcpyAsync(lp_out + q0, dlp, sizeof(double) * nb, cudaMemcpyDeviceToHost, c->stream));
         EPG_CHECK(c, cudaMemcpyAsync(grad_out + (size_t)q0 * p, dg, sizeof(double) * (size_t)nb * p, cudaMemcpyDeviceToHost, c->stream));
         EPG_CHECK(c, cudaStreamSynchronize(c->stream));
     }
+#undef LAUNCH_LD
+    return 0;
+}
+
+int epg_last_plan(epg_ctx* c, int32_t* out, int n) {
+    if (!c->sites || !c->sites->plan[0] || !out || n < 1)
+        return epg_fail_msg(c, "epg_last_plan: no sampling or log-density launch yet");
+    memcpy(out, c->sites->plan, sizeof(int32_t) * std::min(n, EPG_PLAN_FIELDS));
     return 0;
 }
 

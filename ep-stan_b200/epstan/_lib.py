@@ -86,8 +86,14 @@ SYMBOLS = [
                                     _c_double_p, _c_double_p, _c_int64_p, _c_double_p]),
     ('epg_set_option', C.c_int, [C.c_void_p, C.c_char_p, C.c_double]),
     ('epg_num_params', C.c_int, [C.c_void_p, C.c_int]),
-    ('epg_logdensity', C.c_int, [C.c_void_p, C.c_int, C.c_int, _c_double_p, _c_double_p, _c_double_p]),
+    ('epg_logdensity', C.c_int, [C.c_void_p, C.c_int, C.c_int, _c_double_p, _c_double_p, _c_double_p,
+                                 C.c_int, C.c_int]),
+    ('epg_last_plan', C.c_int, [C.c_void_p, _c_int32_p, C.c_int]),
 ]
+
+# fields of epg_last_plan, in order (include/epgpu.h)
+PLAN_FIELDS = ('kernel', 'use_tc', 'chain_pad', 'tc_nst', 'resident', 'R', 'slices', 'NC', 'hot_nvec',
+               'hot_levels', 'omega_smem', 'smem_total')
 
 
 def load():
@@ -417,10 +423,21 @@ class Context:
     def num_params(self, k):
         return int(self._lib.epg_num_params(self._h, k))
 
-    def logdensity(self, k, q):
+    def logdensity(self, k, q, chains=None, ticks=2):
+        """Tilted log-density and gradient of site k at the rows of q, evaluated in batches of `chains` under
+        the launch plan tilted_sample makes for that many chains (None: when the single-box tensor-core pass
+        may serve the sites, the most chains <= 16 at which the sampler keeps it, else 32); the likelihood pass
+        runs `ticks` times before the read-out."""
         q = _f64(np.atleast_2d(q), 'C')
         nq, p = q.shape
         lp = np.empty(nq)
         grad = np.empty((nq, p))
-        self._ck(self._lib.epg_logdensity(self._h, k, nq, _dp(q), _dp(lp), _dp(grad)))
+        self._ck(self._lib.epg_logdensity(self._h, k, nq, _dp(q), _dp(lp), _dp(grad),
+                                          0 if chains is None else int(chains), int(ticks)))
         return lp, grad
+
+    def last_plan(self):
+        """Launch plan of the last tilted_sample or logdensity: a dict over PLAN_FIELDS."""
+        out = np.zeros(len(PLAN_FIELDS), dtype=np.int32)
+        self._ck(self._lib.epg_last_plan(self._h, out.ctypes.data_as(_c_int32_p), len(out)))
+        return dict(zip(PLAN_FIELDS, (int(v) for v in out)))

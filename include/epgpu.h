@@ -271,9 +271,32 @@ int epg_set_option(epg_ctx* ctx, const char* name, double value);
 
 /* Direct evaluation of the tilted log-density and its gradient for site k at
  * `nq` points q [nq][p] (p = epg_num_params); used by the parity tests against
- * the fp64 oracle.  lp_out[nq], grad_out[nq][p]. */
+ * the fp64 oracle.  lp_out[nq], grad_out[nq][p].
+ * The points are evaluated in batches of `chains` (1..32) under the launch plan epg_tilted_sample makes for
+ * that many chains: the same likelihood pass (SIMT, tensor-core or wide tensor-core, including the fall-back
+ * to SIMT when the chain vectors do not fit in shared memory), the same shared-memory layout, ring depth and
+ * chain-vector addressing.  chains <= 0: when the single-box tensor-core pass may serve the sites, the most
+ * chains (<= 16) at which the sampler keeps it; otherwise 32.
+ * `ticks` (>= 1): how many times the likelihood pass runs before the read-out (the sampler runs it once per
+ * gradient evaluation and carries the pipeline state of the tensor-core passes from one to the next). */
 int epg_num_params(epg_ctx* ctx, int k);
-int epg_logdensity(epg_ctx* ctx, int k, int nq, const double* q, double* lp_out, double* grad_out);
+int epg_logdensity(epg_ctx* ctx, int k, int nq, const double* q, double* lp_out, double* grad_out,
+                   int chains, int ticks);
+
+/* Launch plan of the most recent epg_tilted_sample or epg_logdensity, as EPG_PLAN_FIELDS int32 in this order:
+ *   kernel      1 = per-site sampling kernel, 2 = two-sites-per-CTA sampling kernel, 3 = log-density kernel
+ *   use_tc      0 = fp32 SIMT pass, 1 = tensor-core pass (D+1 <= 64, <= 16 chains), 2 = wide tensor-core pass
+ *   chain_pad   SIMT: chains padded to 4, 8, 16 or 32; tensor-core pass: chain columns processed (4, 8 or 16);
+ *               wide pass: 32
+ *   tc_nst      X-tile stages of the tensor-core ring (0 on the SIMT pass)
+ *   resident    SIMT: the design matrix stays in shared memory (1) or is streamed in tiles (0)
+ *   R, slices, NC   SIMT: rows per tile, row slices of the gradient product, chain-column blocks per thread
+ *   hot_nvec, hot_levels   per-chain vectors and tree-stack levels kept in shared memory
+ *   omega_smem  the cavity precision lives in shared memory
+ *   smem_total  dynamic shared memory of the launch (bytes)
+ * Writes min(n, EPG_PLAN_FIELDS) values; fails before the first such call. */
+#define EPG_PLAN_FIELDS 12
+int epg_last_plan(epg_ctx* ctx, int32_t* out, int n);
 
 #ifdef __cplusplus
 }

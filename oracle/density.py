@@ -71,8 +71,9 @@ class TiltedDensity(object):
             etb = q[..., d + J:].reshape(q.shape[:-1] + (J, D))
         return phi, eta, etb
 
-    def lp_grad(self, q):
-        """q: (nq, p) -> (lp (nq,), grad (nq, p))"""
+    def lp_grad(self, q, e_map=None):
+        """q: (nq, p) -> (lp (nq,), grad (nq, p)).  e_map: applied to the residuals e = y - sigmoid(f) before
+        they enter the gradient (e.g. the rounding a kernel stores them with); None: exact fp64."""
         q = np.atleast_2d(np.asarray(q, dtype=np.float64))
         nq = q.shape[0]
         D, J, d = self.D, self.J, self.d
@@ -108,6 +109,8 @@ class TiltedDensity(object):
         with np.errstate(over='ignore', invalid='ignore'):
             lp_lik = np.sum(self.y * f - np.logaddexp(0.0, f), axis=1)
             e = self.y - 1.0 / (1.0 + np.exp(-f))                      # (nq,N)
+        if e_map is not None:
+            e = e_map(e)
         if J == 1:
             s = e.sum(axis=1, keepdims=True)
             g = (e @ self.X)[:, None, :]

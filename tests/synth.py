@@ -43,3 +43,11 @@ def tc_stored_X(X):
     c = X.mean(axis=0).astype(np.float32)
     dev = X.astype(np.float32) - c
     return c.astype(np.float64) + bf16_round(dev)
+
+
+def tc_oracle(model, site):
+    """fp64 oracle of the tensor-core passes (csrc/epg_lik_tc.cuh, epg_lik_tcw.cuh): the design matrix as
+    tc_stored_X holds it, and the residuals E = y - sigmoid(f) rounded to bf16 as the epilogue stores them for
+    the gradient product G = E'X.  Returns lp_grad(q) -> (lp, grad)."""
+    td = oracle_density(model, dict(site, X=tc_stored_X(site['X'])))
+    return lambda q: td.lp_grad(q, e_map=bf16_round)
