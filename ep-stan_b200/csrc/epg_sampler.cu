@@ -64,6 +64,7 @@ struct epg_site_data {
     int param_stats = 0;
     int carry_adapt = 1;                // option "carry_adapt": init_prev runs start from the previous run's adapted metric / step size
     int pp_mode = 0;                    // option "pingpong": 0 never (default), 1 when sites > SMs and L2-resident, 2 always
+    float metric_reg = 1e-3f;           // option "metric_reg": identity weight of the regularised dense_e window estimate
     float* y = nullptr;                 // [N]
     int64_t* row0 = nullptr;            // [K+1]
     int* grp_ptr = nullptr;             // [K+1] offsets into grp_rows
@@ -75,7 +76,7 @@ struct epg_site_data {
     // sampler state
     float* chain_mem = nullptr;         // [K*C][NVEC][P]
     size_t chain_mem_bytes = 0;
-    float* last_q = nullptr;            // [K*C][P] last draw of every chain (init_prev)
+    float* last_q = nullptr;            // [K*C][P] last draw of every chain (init_prev), then last_minv, last_eps, last_metric
     size_t last_q_bytes = 0;
     int last_C = 0;
     float* omega = nullptr;             // [K][d*d] fp32 copy of the cavity precision
@@ -84,6 +85,10 @@ struct epg_site_data {
     size_t out_bytes = 0;
     double* ld_buf = nullptr;           // logdensity staging
     size_t ld_bytes = 0;
+    float* dense = nullptr;             // dense_e state [K*C][dense_floats(P)] (first dense_e run on)
+    size_t dense_bytes = 0;
+    double* dense_ws = nullptr;         // dense_e window-end factorisation scratch [K*C][P][P]
+    size_t dense_ws_bytes = 0;
     int32_t plan[EPG_PLAN_FIELDS] = {}; // launch plan of the last epg_tilted_sample / epg_logdensity (epg_last_plan)
 };
 
@@ -93,6 +98,7 @@ void epg_sites_free(epg_ctx* c) {
     cudaFree(s->xmean); cudaFree(s->gout_w); cudaFree(s->order); cudaFree(s->reinit); cudaFree(s->tstats);
     cudaFree(s->X); cudaFree(s->Xb); cudaFree(s->y); cudaFree(s->row0); cudaFree(s->grp_ptr); cudaFree(s->grp_rows);
     cudaFree(s->chain_mem); cudaFree(s->last_q); cudaFree(s->omega); cudaFree(s->out); cudaFree(s->ld_buf);
+    cudaFree(s->dense); cudaFree(s->dense_ws);
     delete s;
     c->sites = nullptr;
 }
@@ -230,7 +236,11 @@ struct SamplerArgs {
     // chains
     float* chain_mem; float* last_q; int P, C;
     float* last_minv; float* last_eps;  // [K*C][P], [K*C]: adapted metric / step size at the end of the previous run
+    float* last_metric;                 // [K*C]: the metric (EPG_METRIC_*) of that run
     int carry_adapt;                    // init_prev also starts the warm-up from them (option "carry_adapt")
+    int metric;                         // EPG_METRIC_*
+    float* dense; double* dense_ws;     // dense_e: per-chain state (dense_floats) and fp64 scratch [K*C][P][P]
+    float metric_reg;                   // dense_e window estimate: n/(n+5) C + metric_reg 5/(n+5) I
     int iter, warmup, init_mode, max_depth;
     double delta;
     int win_init, win_term, win_base;
@@ -789,8 +799,17 @@ __device__ void likelihood_pass_tcw(const SamplerArgs& a, unsigned char* smem, u
 // the cavity mean live in shared memory; they are then addressed through the __shared__ symbol so that the
 // compiler emits ld.shared / st.shared instead of generic loads (which take the L1TEX path: ~50 cycles more
 // per dependent access, and the chain phase is one long dependency chain).
-template <bool ALLHOT>
+// DENSE = true: the chain runs Stan's dense_e metric; its p x p matrices and the p_sharp vectors of the
+// trajectory live in the dense_e block (global memory), which the diag_e / unit_e instances never touch.
+//   dense block of a chain: [Sigma][U^-1 stored by columns][window co-moment] (P x P each), then
+//   p_sharp of the working point, of the minus end and of the plus end (P each)
+enum { DN_SIGMA = 0, DN_UINV, DN_W2 };
+enum { DV_PSH = 0, DV_PSM, DV_PSP };
+__host__ __device__ inline size_t dense_floats(int P) { return 3 * (size_t)P * P + 3 * (size_t)P; }
+
+template <bool ALLHOT, bool DENSE = false>
 struct ChainCtxT {
+    static constexpr bool kDense = DENSE;
     const SamplerArgs& a;
     int cg;          // global chain index (k_local*C + c)
     int p, d, J, D, lane;
@@ -802,6 +821,10 @@ struct ChainCtxT {
     float* hot;           // this chain's block of shared-memory vectors (hot vectors, then hot stack levels)
     float* cold;          // this chain's vectors in global memory
     uint32_t hot_off, cavc_off, muf_off;      // the same three as byte offsets into dynamic shared memory
+    float* dn;            // dense_e block of this chain (DENSE only)
+    double* ws;           // dense_e fp64 factorisation scratch [P][P] (DENSE only)
+    __device__ __forceinline__ float* dm(int which) const { return dn + (size_t)which * a.P * a.P; }
+    __device__ __forceinline__ float* dv(int which) const { return dn + 3 * (size_t)a.P * a.P + (size_t)which * a.P; }
     __device__ __forceinline__ float* v(int which) const {
         if constexpr (ALLHOT) {
             extern __shared__ __align__(1024) unsigned char smem_dyn[];
@@ -828,10 +851,10 @@ struct ChainCtxT {
         } else return muf_;
     }
 };
-template <bool ALLHOT>
-__device__ __forceinline__ ChainCtxT<ALLHOT> make_chain_ctx(const SamplerArgs& a, const SiteView& sv, int c_local, int p,
-                                                            int d, int J, int D, int lane, uint2 key, const float* om,
-                                                            const float* muf, ChainStack* stk) {
+template <bool ALLHOT, bool DENSE = false>
+__device__ __forceinline__ ChainCtxT<ALLHOT, DENSE> make_chain_ctx(const SamplerArgs& a, const SiteView& sv, int c_local,
+                                                                   int p, int d, int J, int D, int lane, uint2 key,
+                                                                   const float* om, const float* muf, ChainStack* stk) {
     const int cg = sv.k * a.C + c_local;
     float* hot = cvec(a, sv, c_local, 0);    // slot 0 of the chain's shared block (when hot_nvec > 0)
     float* cold = a.chain_mem + (size_t)cg * NVEC * a.P;
@@ -841,7 +864,14 @@ __device__ __forceinline__ ChainCtxT<ALLHOT> make_chain_ctx(const SamplerArgs& a
     const uint32_t hot_off = sv.off + (uint32_t)a.off_hot + (uint32_t)c_local * per_chain * (uint32_t)a.P * 4u;
     const uint32_t cavc_off = sv.off + (uint32_t)a.off_cavc + (uint32_t)(c_local * d) * 4u;
     const uint32_t muf_off = sv.off + (uint32_t)a.off_omega + (uint32_t)(d * d) * 4u;
-    return ChainCtxT<ALLHOT>{a, cg, p, d, J, D, lane, key, om, muf, stk, cavc, hot, cold, hot_off, cavc_off, muf_off};
+    float* dn = nullptr;
+    double* ws = nullptr;
+    if constexpr (DENSE) {
+        dn = a.dense + (size_t)cg * dense_floats(a.P);
+        ws = a.dense_ws + (size_t)cg * a.P * a.P;
+    }
+    return ChainCtxT<ALLHOT, DENSE>{a, cg, p, d, J, D, lane, key, om, muf, stk, cavc, hot, cold, hot_off, cavc_off,
+                                    muf_off, dn, ws};
 }
 
 template <class CX>
@@ -850,10 +880,41 @@ __device__ __forceinline__ void vcopy(const CX& x, int dst, int src) {
     const float4* S_ = reinterpret_cast<const float4*>(x.v(src));
     for (int i = x.lane; 4 * i < x.p; i += 32) D_[i] = S_[i];       // vectors are padded to P (multiple of 32)
 }
+// the same for the p_sharp vectors of the dense_e block
+template <class CX>
+__device__ __forceinline__ void dcopy(const CX& x, int dst, int src) {
+    float4* D_ = reinterpret_cast<float4*>(x.dv(dst));
+    const float4* S_ = reinterpret_cast<const float4*>(x.dv(src));
+    for (int i = x.lane; 4 * i < x.p; i += 32) D_[i] = S_[i];
+}
 
-// kinetic energy 0.5 p' M^-1 p
+// dense_e: out = M v on the chain's warp.  Entry (i, j) of M is stored at M[j P + i] (M symmetric, or stored
+// by columns), so for each j the lanes read P consecutive floats while v_j is a broadcast: p^2/32 FMAs per lane.
+// `upper`: entry (i, j) is zero for j < i, and the sum over j starts at the first row of the lane's chunk.
+// The sum runs over increasing j from 0: for the identity it returns v exactly (the zero terms add +0).
+// v must be visible to the whole warp (written before a __syncwarp) and must not alias out.
+template <class CX>
+__device__ __forceinline__ void warp_matvec(const CX& x, const float* M, const float* v, float* out, bool upper) {
+    const size_t P = x.a.P;
+    for (int i0 = 0; i0 < x.p; i0 += 32) {
+        const int i = i0 + x.lane;                        // (< P: P is a multiple of 32)
+        float acc = 0.0f;
+        for (int j = upper ? i0 : 0; j < x.p; ++j) acc = fmaf(M[(size_t)j * P + i], v[j], acc);
+        if (i < x.p) out[i] = acc;
+    }
+    __syncwarp();
+}
+
+// kinetic energy 0.5 p' M^-1 p  (dense_e: also leaves p_sharp = Sigma p of the working point in DV_PSH)
 template <class CX>
 __device__ __forceinline__ double kinetic(const CX& x, const float* p) {
+    if constexpr (CX::kDense) {
+        float* ps = x.dv(DV_PSH);
+        warp_matvec(x, x.dm(DN_SIGMA), p, ps, false);
+        float s = 0.0f;
+        for (int i = x.lane; i < x.p; i += 32) s = fmaf(ps[i], p[i], s);
+        return 0.5 * warp_sum((double)s);
+    }
     const float* minv = x.v(V_MINV);
     float s = 0.0f;
     for (int i = x.lane; i < x.p; i += 32) s += minv[i] * p[i] * p[i];
@@ -914,11 +975,27 @@ __device__ void leaf_fused(const CX& x, double lp_lik, float eps_signed, double&
             gi = qi - gl[i];
         }
         const float pi = p[i] - 0.5f * eps_signed * gi;
-        const float mp = minv[i] * pi;
-        kin2 = fmaf(mp, pi, kin2);
-        g[i] = gi; p[i] = pi;
-        crho[i] = pi; cpsl[i] = mp;
-        qp_[i] = qi; gp_[i] = gi;
+        if constexpr (CX::kDense) {
+            g[i] = gi; p[i] = pi;
+            crho[i] = pi;
+            qp_[i] = qi; gp_[i] = gi;
+        } else {
+            const float mp = minv[i] * pi;
+            kin2 = fmaf(mp, pi, kin2);
+            g[i] = gi; p[i] = pi;
+            crho[i] = pi; cpsl[i] = mp;
+            qp_[i] = qi; gp_[i] = gi;
+        }
+    }
+    if constexpr (CX::kDense) {          // p_sharp = Sigma p needs all of p: a second pass
+        __syncwarp();
+        float* ps = x.dv(DV_PSH);
+        warp_matvec(x, x.dm(DN_SIGMA), p, ps, false);
+        for (int i = x.lane; i < x.p; i += 32) {
+            const float mp = ps[i];
+            kin2 = fmaf(mp, p[i], kin2);
+            cpsl[i] = mp;
+        }
     }
     // two reductions interleaved
     double a = (double)prior2, b = (double)kin2;
@@ -937,6 +1014,15 @@ __device__ void sample_momentum(const CX& x, ChainS& s) {
     const float* minv = x.v(V_MINV);
     float* p = x.v(V_P);
     const uint32_t ctr = s.rng++;
+    if constexpr (CX::kDense) {
+        // p = U^-1 z with Sigma = U'U, z ~ N(0, I): p ~ N(0, Sigma^-1) (dense_e_metric.hpp sample_p).  z goes
+        // through the minus-end p_sharp, which a transition / step-size trial sets only after this.
+        float* z = x.dv(DV_PSM);
+        for (int i = x.lane; i < x.p; i += 32) z[i] = rng_normal(x.key, ctr, (uint32_t)i);
+        __syncwarp();
+        warp_matvec(x, x.dm(DN_UINV), z, p, true);
+        return;
+    }
     for (int i = x.lane; i < x.p; i += 32) p[i] = rng_normal(x.key, ctr, (uint32_t)i) * rsqrtf(minv[i]);
     __syncwarp();
 }
@@ -945,6 +1031,15 @@ __device__ void sample_momentum(const CX& x, ChainS& s) {
 template <class CX>
 __device__ void leapfrog_begin(const CX& x, float eps_signed) {
     float* q = x.v(V_Q); float* p = x.v(V_P); const float* g = x.v(V_G); const float* minv = x.v(V_MINV);
+    if constexpr (CX::kDense) {          // q += e Sigma p, through the working point's p_sharp (recomputed at the leaf)
+        for (int i = x.lane; i < x.p; i += 32) p[i] = p[i] - 0.5f * eps_signed * g[i];
+        __syncwarp();
+        float* ps = x.dv(DV_PSH);
+        warp_matvec(x, x.dm(DN_SIGMA), p, ps, false);
+        for (int i = x.lane; i < x.p; i += 32) q[i] += eps_signed * ps[i];
+        __syncwarp();
+        return;
+    }
     for (int i = x.lane; i < x.p; i += 32) {
         const float ph = p[i] - 0.5f * eps_signed * g[i];
         p[i] = ph;
@@ -998,6 +1093,7 @@ __device__ void begin_transition(const CX& x, ChainS& s) {
     vcopy(x, V_QM, V_Q); vcopy(x, V_PM, V_P); vcopy(x, V_GM, V_G);
     vcopy(x, V_QP, V_Q); vcopy(x, V_PP, V_P); vcopy(x, V_GP, V_G);
     vcopy(x, V_RHO, V_P);
+    if constexpr (CX::kDense) { dcopy(x, DV_PSM, DV_PSH); dcopy(x, DV_PSP, DV_PSH); }   // (kinetic() set PSH)
     __syncwarp();
     s.lsw = 0.0;
     s.depth = 0;
@@ -1015,6 +1111,63 @@ __device__ void next_window(const SamplerArgs& a, ChainS& s) {
     if (s.win_next == last) return;
     const int boundary = s.win_next + 2 * s.win_size;
     if (boundary >= a.warmup - a.win_term) s.win_next = last;
+}
+
+// dense_e window end (covar_adaptation.hpp learn_covariance + dense_e_metric): from the window's co-moment W2 of
+// n draws, Sigma = n/(n+5) W2/(n-1) + reg 5/(n+5) I, formed and Cholesky-factored (Sigma = L L', U = L') in fp64
+// in the chain's scratch, by the chain's warp.  On success Sigma (fp32, symmetric), U^-1 = (L^-1)' stored by
+// columns and diag(Sigma) in V_MINV are replaced; a non-finite or non-positive pivot leaves all three as they were.
+template <class CX>
+__device__ void dense_window_end(const CX& x, int n) {
+    const int p = x.p, lane = x.lane;
+    const size_t P = x.a.P;
+    double* A = x.ws;
+    const float* w2 = x.dm(DN_W2);
+    const double sc = (double)n / ((double)n + 5.0) / ((double)n - 1.0);
+    const double reg = (double)x.a.metric_reg * (5.0 / ((double)n + 5.0));
+    // lower triangle (Stan's LLT reads the lower triangle of the estimate too)
+    for (int i = 0; i < p; ++i)
+        for (int j = lane; j <= i; j += 32) A[i * P + j] = sc * (double)w2[i * P + j] + (i == j ? reg : 0.0);
+    __syncwarp();
+    // right-looking Cholesky, lane r owns rows r, r + 32, ...
+    bool ok = true;
+    for (int k = 0; k < p; ++k) {
+        const double piv = A[k * P + k];
+        if (!(piv > 0.0 && isfinite(piv))) { ok = false; break; }       // (the same value on every lane)
+        const double lkk = sqrt(piv), rl = 1.0 / lkk;
+        for (int i = k + 1 + lane; i < p; i += 32) A[i * P + k] *= rl;
+        __syncwarp();
+        if (lane == 0) A[k * P + k] = lkk;
+        for (int i = k + 1 + lane; i < p; i += 32) {
+            const double lik = A[i * P + k];
+            for (int j = k + 1; j <= i; ++j) A[i * P + j] -= lik * A[j * P + k];
+        }
+        __syncwarp();
+    }
+    __syncwarp();
+    if (!ok) return;
+    // L^-1 column by column (lane r: columns r, r + 32, ...): L x = e_j, x_i (i > j) kept in the free upper
+    // triangle A[j][i]
+    for (int j = lane; j < p; j += 32) {
+        const double xj = 1.0 / A[j * P + j];
+        for (int i = j + 1; i < p; ++i) {
+            double acc = A[i * P + j] * xj;
+            for (int k = j + 1; k < i; ++k) acc += A[i * P + k] * A[j * P + k];
+            A[j * P + i] = -acc / A[i * P + i];
+        }
+    }
+    __syncwarp();
+    // U^-1 (i, j) = L^-1 (j, i), nonzero for i <= j, stored at ui[j P + i]; Sigma recomputed from W2
+    float* sig = x.dm(DN_SIGMA); float* ui = x.dm(DN_UINV); float* minv = x.v(V_MINV);
+    for (int j = 0; j < p; ++j)
+        for (int i = lane; i < p; i += 32) {
+            ui[j * P + i] = i < j ? (float)A[i * P + j] : (i == j ? (float)(1.0 / A[i * P + i]) : 0.0f);
+            const int r = i > j ? i : j, c = i > j ? j : i;
+            sig[j * P + i] = (float)(sc * (double)w2[r * P + c] + (i == j ? reg : 0.0));
+        }
+    __syncwarp();
+    for (int i = lane; i < p; i += 32) minv[i] = sig[i * P + i];
+    __syncwarp();
 }
 
 // bookkeeping at the end of a transition; returns with the next request issued
@@ -1036,10 +1189,28 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
         const double x_eta = pow((double)s.da_count, -0.75);
         s.x_bar = (1.0 - x_eta) * s.x_bar + x_eta * xx;
         s.eps = (float)exp(xx);
-        // ---- variance windows (var_adaptation::learn_variance) ----
-        const bool in_win = a.warmup >= 20 && s.win_count >= a.win_init &&
+        // ---- variance windows (var_adaptation::learn_variance; dense_e: covar_adaptation; unit_e: none) ----
+        const bool windows = a.warmup >= 20 && a.metric != EPG_METRIC_UNIT;
+        const bool in_win = windows && s.win_count >= a.win_init &&
                             s.win_count < a.warmup - a.win_term && s.win_count != a.warmup;
-        if (in_win) {
+        if (CX::kDense && in_win) {
+            // Welford co-moment (welford_covar_estimator): m += d/n, W2 += (q - m) d'.  d and q - m go through the
+            // p_sharp vectors of the ends, which the finished transition no longer needs.
+            s.w_n += 1;
+            float* wm = x.v(V_WMEAN); float* dl = x.dv(DV_PSM); float* dq = x.dv(DV_PSP);
+            for (int i = x.lane; i < x.p; i += 32) {
+                const float dlt = qs[i] - wm[i];
+                wm[i] += dlt / (float)s.w_n;
+                dl[i] = dlt; dq[i] = qs[i] - wm[i];
+            }
+            __syncwarp();
+            float* w2 = x.dm(DN_W2);
+            for (int i = 0; i < x.p; ++i) {
+                const float di = dq[i];
+                for (int j = x.lane; j < x.p; j += 32) w2[(size_t)i * a.P + j] += di * dl[j];
+            }
+            __syncwarp();
+        } else if (in_win) {
             s.w_n += 1;
             float* wm = x.v(V_WMEAN); float* w2 = x.v(V_WM2);
             for (int i = x.lane; i < x.p; i += 32) {
@@ -1048,8 +1219,18 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
                 w2[i] += (qs[i] - wm[i]) * dlt;
             }
         }
-        const bool win_end = a.warmup >= 20 && s.win_count == s.win_next && s.win_count != a.warmup;
-        if (win_end) {
+        const bool win_end = windows && s.win_count == s.win_next && s.win_count != a.warmup;
+        if (CX::kDense && win_end) {
+            next_window(a, s);
+            dense_window_end(x, s.w_n);
+            float* wm = x.v(V_WMEAN); float* w2 = x.dm(DN_W2);
+            for (int i = x.lane; i < x.p; i += 32) wm[i] = 0.0f;
+            for (int i = 0; i < x.p; ++i)
+                for (int j = x.lane; j < x.p; j += 32) w2[(size_t)i * a.P + j] = 0.0f;
+            __syncwarp();
+            s.w_n = 0;
+            restart_ss = true;
+        } else if (win_end) {
             next_window(a, s);
             const float n = (float)s.w_n;
             float* minv = x.v(V_MINV); float* wm = x.v(V_WMEAN); float* w2 = x.v(V_WM2);
@@ -1122,7 +1303,7 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
         float* lm = a.last_minv + (size_t)x.cg * a.P;
         const float* minv = x.v(V_MINV);
         for (int i = x.lane; i < x.p; i += 32) { lq[i] = qs[i]; lm[i] = minv[i]; }
-        if (x.lane == 0) a.last_eps[x.cg] = s.eps;
+        if (x.lane == 0) { a.last_eps[x.cg] = s.eps; a.last_metric[x.cg] = (float)a.metric; }
         s.phase = PH_DONE;
         return;
     }
@@ -1248,6 +1429,17 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
         float* crho = x.v(V_CRHO); float* cpsl = x.v(V_CPSL);
         const float* p = x.v(V_P); const float* minv = x.v(V_MINV);
         float d1 = 0.0f, d2 = 0.0f;
+        if constexpr (CX::kDense) {
+            const float* ps = x.dv(DV_PSH);       // p_sharp of the new leaf (leaf_fused)
+            for (int i = x.lane; i < x.p; i += 32) {
+                const float rs = lrho[i] + crho[i];
+                crho[i] = rs;
+                const float pl = lpsl[i];
+                cpsl[i] = pl;
+                d1 += pl * rs;
+                d2 = fmaf(ps[i], rs, d2);
+            }
+        } else
         for (int i = x.lane; i < x.p; i += 32) {
             const float rs = lrho[i] + crho[i];
             crho[i] = rs;
@@ -1288,6 +1480,7 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
     // ---- the subtree of 2^depth leaves is complete and valid ----
     if (s.sign > 0) { vcopy(x, V_QP, V_Q); vcopy(x, V_PP, V_P); vcopy(x, V_GP, V_G); }
     else            { vcopy(x, V_QM, V_Q); vcopy(x, V_PM, V_P); vcopy(x, V_GM, V_G); }
+    if constexpr (CX::kDense) dcopy(x, s.sign > 0 ? DV_PSP : DV_PSM, DV_PSH);
     s.depth += 1;
     bool take = s.cur_lsw > s.lsw;
     if (!take) take = rng_uniform(x.key, s.rng) < __expf((float)(s.cur_lsw - s.lsw));
@@ -1298,6 +1491,15 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
     {
         float* rho = x.v(V_RHO); const float* crho = x.v(V_CRHO);
         const float* pm = x.v(V_PM); const float* pp = x.v(V_PP); const float* minv = x.v(V_MINV);
+        if constexpr (CX::kDense) {
+            const float* psm = x.dv(DV_PSM); const float* psp = x.dv(DV_PSP);
+            for (int i = x.lane; i < x.p; i += 32) {
+                const float r = rho[i] + crho[i];
+                rho[i] = r;
+                d1 = fmaf(psm[i], r, d1);
+                d2 = fmaf(psp[i], r, d2);
+            }
+        } else
         for (int i = x.lane; i < x.p; i += 32) {
             const float r = rho[i] + crho[i];
             rho[i] = r;
@@ -1337,9 +1539,10 @@ __device__ __forceinline__ void init_chains(const SamplerArgs& a, const SiteView
         // distribution of a site changes little between EP iterations, while a unit metric makes the first
         // 90 % of every warm-up crawl at the scale of the tightest cavity direction with saturated trees.
         // A re-initialised site (mode 3) starts from the conditional cavity variances instead.
+        // (only from a run of the same metric: a diag_e metric is no starting point for dense_e, nor vice versa)
         float eps0 = 1.0f;
         bool carried = false;
-        if (im == 2 && a.carry_adapt) {
+        if (im == 2 && a.carry_adapt && a.last_metric[cg] == (float)a.metric) {
             const float e = a.last_eps[cg];
             if (e > 0.0f && isfinite(e)) { eps0 = e; carried = true; }     // (written together with last_minv)
         }
@@ -1354,9 +1557,10 @@ __device__ __forceinline__ void init_chains(const SamplerArgs& a, const SiteView
             s.win_next = a.win_init + a.win_base - 1;
             s.win_size = a.win_base;
         }
-        const int vecs[] = {V_WMEAN, V_WM2, V_RS0, V_RQ0, V_RS1, V_RQ1};
-        for (int i = lane; i < a.P; i += 32) {
+        // starting inverse metric, element i of the diagonal (unit_e: always 1)
+        auto start_minv = [&](int i) -> float {
             float mv = 1.0f;
+            if (a.metric == EPG_METRIC_UNIT) return mv;
             if (carried) {
                 const float v = a.last_minv[(size_t)cg * a.P + i];
                 if (v > 0.0f && isfinite(v)) mv = v;
@@ -1364,20 +1568,42 @@ __device__ __forceinline__ void init_chains(const SamplerArgs& a, const SiteView
                 const double om = a.cavQ[(size_t)sv.k * a.d * a.d + (size_t)i * a.d + i];
                 if (om > 0.0 && isfinite(om)) mv = (float)(1.0 / om);
             }
+            return mv;
+        };
+        const int vecs[] = {V_WMEAN, V_WM2, V_RS0, V_RQ0, V_RS1, V_RQ1};
+        for (int i = lane; i < a.P; i += 32) {
+            const float mv = start_minv(i);
             cvec(a, sv, c, V_MINV)[i] = mv;
             for (int v = 0; v < 6; ++v) cvec(a, sv, c, vecs[v])[i] = 0.0f;
+        }
+        if (a.metric == EPG_METRIC_DENSE) {
+            // a carried chain keeps Sigma and U^-1 of its previous (dense_e) run; otherwise diagonal: Sigma = the
+            // starting diagonal above, U^-1 = its inverse square root
+            float* dn = a.dense + (size_t)cg * dense_floats(a.P);
+            const size_t PP = (size_t)a.P * a.P;
+            for (int i = 0; i < a.P; ++i) {
+                const float mv = carried ? 0.0f : start_minv(i);
+                for (int j = lane; j < a.P; j += 32) {
+                    if (!carried) {
+                        dn[DN_SIGMA * PP + (size_t)i * a.P + j] = i == j ? mv : 0.0f;
+                        dn[DN_UINV * PP + (size_t)i * a.P + j] = i == j ? (float)(1.0 / sqrt((double)mv)) : 0.0f;
+                    }
+                    dn[DN_W2 * PP + (size_t)i * a.P + j] = 0.0f;
+                }
+            }
         }
     }
 }
 
 // one chain phase of a site: every chain advances to its next gradient request; warp w of nw
-template <bool ALLHOT>
+template <bool ALLHOT, bool DENSE = false>
 __device__ __forceinline__ void chain_phase(const SamplerArgs& a, const SiteView& sv, ChainS* cs, ChainStack* cstk,
                                             const double* lp_lik, int* n_active, int p, int J, uint32_t site_seed,
                                             const float* om, const float* muf, int w, int nw, int lane) {
     for (int c = w; c < a.C; c += nw) {
-        const ChainCtxT<ALLHOT> x = make_chain_ctx<ALLHOT>(a, sv, c, p, a.d, J, a.D, lane,
-                                                           make_uint2(site_seed, (uint32_t)c), om, muf, cstk + c);
+        const ChainCtxT<ALLHOT, DENSE> x = make_chain_ctx<ALLHOT, DENSE>(a, sv, c, p, a.d, J, a.D, lane,
+                                                                         make_uint2(site_seed, (uint32_t)c), om, muf,
+                                                                         cstk + c);
         ChainS s = cs[c];                  // private copy: every lane runs the same scalar code
         const int before = s.phase;
         chain_step(x, s, lp_lik[c], c, sv.k);
@@ -1487,7 +1713,8 @@ __device__ void site_analytics(const SamplerArgs& a, const SiteView& sv, const C
 // the persistent sampling kernel: one CTA per site
 // ---------------------------------------------------------------------------
 // TCM 0: fp32 SIMT likelihood pass (NTHR threads); 1: tensor-core pass, 2: wide tensor-core pass (tc::NTHREADS threads)
-template <int CP, int TCM>
+// DENSE: the dense_e chain phase (separate instances, so that the diag_e / unit_e ones carry none of its code)
+template <int CP, int TCM, bool DENSE>
 __global__ void __launch_bounds__(TCM ? tc::NTHREADS : NTHR, 1)
 k_nuts(const SamplerArgs a, const __grid_constant__ CUtensorMap tmap) {
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -1542,7 +1769,7 @@ k_nuts(const SamplerArgs a, const __grid_constant__ CUtensorMap tmap) {
     long long clk_chain = 0, clk_lik = 0, n_ticks = 0;
     for (;;) {
         const long long tk0 = clock64();
-        if (worker) chain_phase<USE_TC>(a, sv, cs, cstk, lp_lik, &n_active, p, J, site_seed, om, muf, warp, NWARP, lane);
+        if (worker) chain_phase<USE_TC, DENSE>(a, sv, cs, cstk, lp_lik, &n_active, p, J, site_seed, om, muf, warp, NWARP, lane);
         __threadfence_block();
         __syncthreads();
         if (n_active <= 0) break;
@@ -1578,6 +1805,7 @@ struct PPSlot {
 };
 __device__ __forceinline__ void chain_group_sync() { asm volatile("bar.sync 2, %0;\n" ::"n"(32 * PP_NCW) : "memory"); }
 
+template <bool DENSE>
 __global__ void __launch_bounds__(PP_THREADS, 1)
 k_nuts_pp(const SamplerArgs a, const __grid_constant__ CUtensorMap tmap, int n_sites, int* queue) {
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -1644,7 +1872,8 @@ k_nuts_pp(const SamplerArgs a, const __grid_constant__ CUtensorMap tmap, int n_s
                 }
                 const long long t0 = clock64();
                 const SiteView sv{sm, S.k, (uint32_t)((size_t)sc * a.site_stride)};
-                chain_phase<true>(a, sv, cs, cstk, lp_lik[sc], &S.n_active, S.p, 1, S.seed, om, om + d * d, cw, PP_NCW, lane);
+                chain_phase<true, DENSE>(a, sv, cs, cstk, lp_lik[sc], &S.n_active, S.p, 1, S.seed, om, om + d * d, cw,
+                                         PP_NCW, lane);
                 __threadfence_block();
                 chain_group_sync();
                 if (ct == 0) { S.clk_chain += clock64() - t0; S.n_ticks += 1; }
@@ -2040,6 +2269,11 @@ int epg_set_option(epg_ctx* c, const char* name, double value) {
         c->sites->carry_adapt = value != 0.0;
         return 0;
     }
+    if (strcmp(name, "metric_reg") == 0) {
+        if (!c->sites) return epg_fail_msg(c, "epg_set_option(metric_reg): upload the sites first");
+        c->sites->metric_reg = (float)value;
+        return 0;
+    }
     if (strcmp(name, "pingpong") == 0) {
         if (!c->sites) return epg_fail_msg(c, "epg_set_option(pingpong): upload the sites first");
         c->sites->pp_mode = (int)value;
@@ -2067,8 +2301,8 @@ static int fill_args(epg_ctx* c, SamplerArgs& a, int C, int CP, int n_sites = 1,
         EPG_CHECK(c, cudaMalloc((void**)&s->chain_mem, need));
         s->chain_mem_bytes = need;
     }
-    const size_t n_lq = (size_t)c->K * C * s->Pmax;               // last_q | last_minv | last_eps
-    const size_t need_lq = sizeof(float) * (2 * n_lq + (size_t)c->K * C);
+    const size_t n_lq = (size_t)c->K * C * s->Pmax;               // last_q | last_minv | last_eps | last_metric
+    const size_t need_lq = sizeof(float) * (2 * n_lq + 2 * (size_t)c->K * C);
     if (need_lq > s->last_q_bytes || s->last_C != C) {
         if (s->last_q) cudaFree(s->last_q);
         s->last_q = nullptr; s->last_q_bytes = 0;
@@ -2080,6 +2314,8 @@ static int fill_args(epg_ctx* c, SamplerArgs& a, int C, int CP, int n_sites = 1,
     EPG_CHECK(c, epg_reserve((void**)&s->out, &s->out_bytes, sizeof(double) * (size_t)c->K * 8 + sizeof(uint32_t) * ((size_t)c->K + 4)));
     a.chain_mem = s->chain_mem; a.last_q = s->last_q; a.omega = s->omega; a.out = s->out;
     a.last_minv = s->last_q + n_lq; a.last_eps = s->last_q + 2 * n_lq; a.carry_adapt = s->carry_adapt;
+    a.last_metric = a.last_eps + (size_t)c->K * C;
+    a.metric_reg = s->metric_reg;
     a.tstats = nullptr;
     if (s->param_stats) {
         EPG_CHECK(c, epg_reserve((void**)&s->tstats, &s->tstats_bytes, sizeof(double) * (size_t)c->K * 2 * s->Pmax));
@@ -2145,6 +2381,8 @@ int epg_tilted_sample(epg_ctx* c, int k0, int k1, const uint32_t* seeds, const e
     if (o->chains < 1 || o->chains > 32) return epg_fail_msg(c, "chains must be in 1..32");
     if (o->thin != 1) return epg_fail_msg(c, "only thin=1 is supported");
     if (o->iter < 1) return epg_fail_msg(c, "iter must be positive");
+    if (o->metric < EPG_METRIC_DIAG || o->metric > EPG_METRIC_UNIT)
+        return epg_fail_msg(c, "metric must be 0 (diag_e), 1 (dense_e) or 2 (unit_e)");
     const int warm = o->warmup < 0 ? o->iter / 2 : o->warmup;
     if (warm >= o->iter) return epg_fail_msg(c, "warmup must be smaller than iter");
     const int C = o->chains, CP = pad_chains(C);
@@ -2156,6 +2394,15 @@ int epg_tilted_sample(epg_ctx* c, int k0, int k1, const uint32_t* seeds, const e
     memset(&a, 0, sizeof(a));
     if (int rc = fill_args(c, a, C, CP, k1 - k0, true)) return rc;
     a.iter = o->iter; a.warmup = warm; a.init_mode = o->init_mode;
+    a.metric = o->metric;
+    if (a.metric == EPG_METRIC_DENSE) {
+        // (allocated with the first dense_e run; a larger chain count reallocates them, and the carried state with
+        //  them, but then last_q is reallocated and zeroed as well, so nothing is carried)
+        const size_t nch = (size_t)c->K * C;
+        EPG_CHECK(c, epg_reserve((void**)&s->dense, &s->dense_bytes, sizeof(float) * nch * dense_floats(s->Pmax)));
+        EPG_CHECK(c, epg_reserve((void**)&s->dense_ws, &s->dense_ws_bytes, sizeof(double) * nch * s->Pmax * s->Pmax));
+        a.dense = s->dense; a.dense_ws = s->dense_ws;
+    }
     a.max_depth = o->max_treedepth > 0 ? std::min(o->max_treedepth, MAXDEPTH_CAP) : 10;
     a.delta = o->adapt_delta > 0 ? o->adapt_delta : 0.8;
     // Stan 2.17 windowed_adaptation defaults (75 / 50 / 25) and their rescaling
@@ -2196,18 +2443,21 @@ int epg_tilted_sample(epg_ctx* c, int k0, int k1, const uint32_t* seeds, const e
     EPG_CHECK(c, cudaEventCreate(&e0));
     EPG_CHECK(c, cudaEventCreate(&e1));
     EPG_CHECK(c, cudaEventRecord(e0, c->stream));
-#define LAUNCH_NUTS(CPV, TC)                                                      \
+    const bool dense = a.metric == EPG_METRIC_DENSE;
+#define LAUNCH_NUTS_M(CPV, TC, DN)                                                \
     {                                                                             \
-        EPG_CHECK(c, set_smem_attr(k_nuts<CPV, TC>, a.smem_total));               \
-        k_nuts<CPV, TC><<<k1 - k0, TC ? tc::NTHREADS : NTHR, a.smem_total, c->stream>>>(a, s->tmap); \
+        EPG_CHECK(c, set_smem_attr(k_nuts<CPV, TC, DN>, a.smem_total));           \
+        k_nuts<CPV, TC, DN><<<k1 - k0, TC ? tc::NTHREADS : NTHR, a.smem_total, c->stream>>>(a, s->tmap); \
     }
+#define LAUNCH_NUTS(CPV, TC) { if (dense) LAUNCH_NUTS_M(CPV, TC, true) else LAUNCH_NUTS_M(CPV, TC, false) }
     if (a.pp) {
         int* queue = reinterpret_cast<int*>(dseeds + c->K);
         EPG_CHECK(c, cudaMemsetAsync(queue, 0, sizeof(int), c->stream));
-        EPG_CHECK(c, set_smem_attr(k_nuts_pp, a.smem_total));
+        auto kpp = dense ? k_nuts_pp<true> : k_nuts_pp<false>;
+        EPG_CHECK(c, set_smem_attr(kpp, a.smem_total));
         int grid = (k1 - k0) > c->num_sms ? c->num_sms : (k1 - k0 + 1) / 2;     // (forced mode: two sites per CTA)
         if (const char* e = getenv("EPGPU_PP_GRID")) grid = std::max(1, std::min(atoi(e), k1 - k0));
-        k_nuts_pp<<<grid, PP_THREADS, a.smem_total, c->stream>>>(a, s->tmap, k1 - k0, queue);
+        kpp<<<grid, PP_THREADS, a.smem_total, c->stream>>>(a, s->tmap, k1 - k0, queue);
     }
     else if (a.use_tc == 2) LAUNCH_NUTS(32, 2)
     else if (a.use_tc) LAUNCH_NUTS(32, 1)
@@ -2298,6 +2548,30 @@ int epg_get_adapt(epg_ctx* c, int k, float* minv_out, float* eps_out) {
     EPG_CHECK(c, cudaStreamSynchronize(c->stream));
     if (minv_out) EPG_CHECK(c, cudaMemcpy(minv_out, s->last_q + n_lq + (size_t)k * C * s->Pmax, sizeof(float) * (size_t)C * s->Pmax, cudaMemcpyDeviceToHost));
     if (eps_out) EPG_CHECK(c, cudaMemcpy(eps_out, s->last_q + 2 * n_lq + (size_t)k * C, sizeof(float) * C, cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+int epg_get_metric(epg_ctx* c, int k, float* out) {
+    if (!c->sites || k < 0 || k >= c->K || !c->sites->last_q || c->sites->last_C < 1 || !out)
+        return epg_fail_msg(c, "epg_get_metric: no finished sampling run");
+    epg_site_data* s = c->sites;
+    const int C = s->last_C;
+    const size_t P = s->Pmax, n_lq = (size_t)c->K * C * P;
+    std::vector<float> minv((size_t)C * P), met(C);
+    EPG_CHECK(c, cudaStreamSynchronize(c->stream));
+    EPG_CHECK(c, cudaMemcpy(minv.data(), s->last_q + n_lq + (size_t)k * C * P, sizeof(float) * minv.size(), cudaMemcpyDeviceToHost));
+    EPG_CHECK(c, cudaMemcpy(met.data(), s->last_q + 2 * n_lq + (size_t)c->K * C + (size_t)k * C, sizeof(float) * C,
+                            cudaMemcpyDeviceToHost));
+    for (int ch = 0; ch < C; ++ch) {
+        float* o = out + (size_t)ch * P * P;
+        if (met[ch] == (float)EPG_METRIC_DENSE && s->dense) {
+            const float* src = s->dense + ((size_t)k * C + ch) * dense_floats((int)P) + DN_SIGMA * P * P;
+            EPG_CHECK(c, cudaMemcpy(o, src, sizeof(float) * P * P, cudaMemcpyDeviceToHost));
+        } else {
+            std::fill(o, o + P * P, 0.0f);
+            for (size_t i = 0; i < P; ++i) o[i * P + i] = minv[(size_t)ch * P + i];
+        }
+    }
     return 0;
 }
 

@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(os.path.dirname(_HERE), 'libepgpu.so')
 XCHG_SLOTS = 64           # EPG_XCHG_SLOTS: caller-defined doubles at the end of DSUM
 MODEL_IDS = {'m1b': 1, 'm2b': 2, 'm3b': 3, 'm4b': 4, 'm5b': 5}
 PREC_ESTIM = {'sample': 0, 'olse': 1}
+METRICS = {'diag_e': 0, 'dense_e': 1, 'unit_e': 2}     # enum epg_metric (Stan's `metric` names)
 
 _c_double_p = C.POINTER(C.c_double)
 _c_int32_p = C.POINTER(C.c_int32)
@@ -27,7 +28,7 @@ _c_uint32_p = C.POINTER(C.c_uint32)
 class SamplerOpts(C.Structure):
     _fields_ = [('chains', C.c_int32), ('iter', C.c_int32), ('warmup', C.c_int32),
                 ('thin', C.c_int32), ('init_mode', C.c_int32), ('max_treedepth', C.c_int32),
-                ('adapt_delta', C.c_double), ('reserved', C.c_int32 * 8)]
+                ('adapt_delta', C.c_double), ('metric', C.c_int32), ('reserved', C.c_int32 * 7)]
 
 
 class EpgError(RuntimeError):
@@ -58,6 +59,7 @@ SYMBOLS = [
     ('epg_get_param_stats', C.c_int, [C.c_void_p, C.c_int, C.c_int, _c_double_p, _c_double_p]),
     ('epg_max_params', C.c_int, [C.c_void_p]),
     ('epg_get_adapt', C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
+    ('epg_get_metric', C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_float)]),
     ('epg_update_partial', C.c_int, [C.c_void_p, C.c_double]),
     ('epg_update_finish', C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     ('epg_accept', C.c_int, [C.c_void_p]),
@@ -305,6 +307,14 @@ class Context:
                                          eps.ctypes.data_as(C.POINTER(C.c_float))))
         return minv, eps
 
+    def get_metric(self, k, chains):
+        """inverse metric [chains, Pmax, Pmax] (fp32) site k's chains ended their last run with: diagonal
+        (diag_e), the identity (unit_e) or the adapted full matrix (dense_e)"""
+        P = int(self._lib.epg_max_params(self._h))
+        out = np.empty((chains, P, P), dtype=np.float32)
+        self._ck(self._lib.epg_get_metric(self._h, int(k), out.ctypes.data_as(C.POINTER(C.c_float))))
+        return out
+
     def update_partial(self, df):
         self._ck(self._lib.epg_update_partial(self._h, float(df)))
 
@@ -402,12 +412,16 @@ class Context:
             None if jk is None else jk.ctypes.data_as(_c_int32_p)))
 
     def tilted_sample(self, seeds, chains, iter, warmup=None, init_mode=0, k0=0, k1=None,
-                      max_treedepth=10, adapt_delta=0.8):
+                      max_treedepth=10, adapt_delta=0.8, metric='diag_e'):
+        """metric: 'diag_e' (Stan's default), 'dense_e' or 'unit_e'"""
         k1 = self.K if k1 is None else k1
+        if metric not in METRICS:
+            raise ValueError("metric must be one of %s, not %r" % (sorted(METRICS), metric))
         seeds = np.ascontiguousarray(seeds, dtype=np.uint32)
         assert seeds.size == k1 - k0
         opts = SamplerOpts(chains=chains, iter=iter, warmup=-1 if warmup is None else warmup, thin=1,
-                           init_mode=init_mode, max_treedepth=max_treedepth, adapt_delta=adapt_delta)
+                           init_mode=init_mode, max_treedepth=max_treedepth, adapt_delta=adapt_delta,
+                           metric=METRICS[metric])
         msteps = np.empty(k1 - k0)
         mrhat = np.empty(k1 - k0)
         nleap = np.empty(k1 - k0, dtype=np.int64)

@@ -101,7 +101,8 @@ class Worker(object):
         'thin'            : 1,
         'init'            : 'random',
         # extension (PyStan's own `sampling` keyword, which the reference never sets): NUTS controls of the
-        # built-in sampler, {'max_treedepth': int, 'adapt_delta': float}; None = Stan's defaults (10, 0.8)
+        # built-in sampler, {'max_treedepth': int, 'adapt_delta': float, 'metric': 'diag_e' | 'dense_e' |
+        # 'unit_e'}; None = Stan's defaults (10, 0.8, 'diag_e')
         'control'         : None
     }
 
@@ -164,8 +165,13 @@ class Worker(object):
             if self.stan_params['init'] not in ('random', '0', 0):
                 raise ValueError("built-in sampler supports init 'random' or '0' only")
             ctl = self.stan_params['control']
-            if ctl is not None and (not isinstance(ctl, dict) or set(ctl) - {'max_treedepth', 'adapt_delta'}):
-                raise ValueError("built-in sampler: `control` may hold 'max_treedepth' and 'adapt_delta' only")
+            if ctl is not None and (not isinstance(ctl, dict) or
+                                    set(ctl) - {'max_treedepth', 'adapt_delta', 'metric'}):
+                raise ValueError("built-in sampler: `control` may hold 'max_treedepth', 'adapt_delta' and "
+                                 "'metric' only")
+            if ctl is not None and ctl.get('metric', 'diag_e') not in _lib.METRICS:
+                raise ValueError("built-in sampler: control['metric'] must be one of {} (got {!r})".format(
+                    sorted(_lib.METRICS), ctl['metric']))
         self.init_prev = options['init_prev']
         self.adapt_prev = bool(options['adapt_prev'])
         self.init_orig = self.stan_params['init']

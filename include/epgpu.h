@@ -220,8 +220,22 @@ typedef struct epg_sampler_opts {
     int32_t init_mode;     /* 0: 'random' U(-2,2); 1: zeros; 2: previous last draws (init_prev, method.py:404-406) */
     int32_t max_treedepth; /* Stan default 10 */
     double adapt_delta;    /* Stan default 0.8 */
-    int32_t reserved[8];
+    int32_t metric;        /* EPG_METRIC_*; 0 (diag_e) is Stan's default.  Other values: the call fails (< 0) */
+    int32_t reserved[7];
 } epg_sampler_opts;
+
+/* Euclidean metrics of the sampler (PyStan `control={'metric': ...}`), with Sigma the p x p inverse metric:
+ *   EPG_METRIC_DIAG  diag_e: Sigma diagonal, adapted from the variances of the draws of each warm-up window
+ *                    (stan/mcmc/hmc/hamiltonians/diag_e_metric.hpp, stan/mcmc/var_adaptation.hpp);
+ *   EPG_METRIC_DENSE dense_e: Sigma = U'U full, momentum p = U^-1 z (z ~ N(0, I)), kinetic energy p'Sigma p / 2,
+ *                    position update q += eps Sigma p; each window end sets Sigma = n/(n+5) C + 1e-3 5/(n+5) I from
+ *                    the window's sample covariance C (stan/mcmc/hmc/hamiltonians/dense_e_metric.hpp,
+ *                    stan/mcmc/covar_adaptation.hpp).  A window whose Sigma has no Cholesky factor (fp64) leaves
+ *                    the chain's previous Sigma in place;
+ *   EPG_METRIC_UNIT  unit_e: Sigma = I, step-size adaptation only (stan/mcmc/hmc/nuts/adapt_unit_e_nuts.hpp).
+ * carry_adapt carries Sigma and the step size over only between runs of a chain with the same metric; otherwise
+ * the warm-up starts from Sigma = I and step size 1. */
+enum epg_metric { EPG_METRIC_DIAG = 0, EPG_METRIC_DENSE = 1, EPG_METRIC_UNIT = 2 };
 
 /* Runs adaptive NUTS for sites [k0,k1) x chains on their tilted densities
  * (cavity from EPG_CAVQ/EPG_CAVM x site likelihood), leaves the post-warm-up
@@ -255,6 +269,11 @@ int epg_max_params(epg_ctx* ctx);
 /* Diagnostics: the diagonal inverse metric [chains][Pmax] (fp32, Pmax = the largest epg_num_params of the
  * context) and the step size [chains] site k's chains ended their last run with (what carry_adapt carries over). */
 int epg_get_adapt(epg_ctx* ctx, int k, float* minv_out, float* eps_out);
+/* The inverse metric Sigma site k's chains ended their last run with, as full matrices [chains][Pmax][Pmax]
+ * (fp32, row-major, Pmax = epg_max_params; entries beyond the site's epg_num_params are undefined): diag_e gives
+ * a diagonal matrix, unit_e the identity, dense_e the adapted Sigma (whose diagonal epg_get_adapt returns).
+ * Fails before the first sampling run. */
+int epg_get_metric(epg_ctx* ctx, int k, float* out);
 
 /* Options.  "carry_adapt" (default 1): a run with init_mode 2 (init_prev) starts its warm-up from the metric
  * and step size the previous run of the same chain ended with, instead of Stan's unit metric and step size 1
@@ -266,7 +285,9 @@ int epg_get_adapt(epg_ctx* ctx, int k, float* minv_out, float* eps_out);
  * sites than SMs and design matrices that stay L2-resident, run the persistent
  * two-sites-per-CTA kernel (likelihood pass of one site overlapped with the chain
  * phase of the other); 2 = always; 0 = never (measured gain on B200 is <= 15 %).
- * Draws do not depend on these two kernels' choice.  Call after epg_upload_sites. */
+ * Draws do not depend on these two kernels' choice.  "metric_reg" (default 1e-3, Stan's value): the weight of
+ * the identity in the regularised dense_e window estimate (n/(n+5) C + metric_reg 5/(n+5) I); a value <= 0
+ * lets a window that is (numerically) singular fail its factorisation.  Call after epg_upload_sites. */
 int epg_set_option(epg_ctx* ctx, const char* name, double value);
 
 /* Direct evaluation of the tilted log-density and its gradient for site k at
