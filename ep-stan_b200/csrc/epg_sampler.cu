@@ -33,6 +33,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <cmath>
 #include <vector>
 
 #define NTHR 256
@@ -56,6 +57,9 @@ struct epg_site_data {
     std::vector<double> h_cost;         //     previous run, h_cost) first, so that stragglers do not start last
     unsigned char* reinit = nullptr;    // [K] 1: the next init_prev run starts this site's chains at random (epg_reinit_sites)
     std::vector<unsigned char> h_reinit;
+    float* inits = nullptr;             // [K][inits_C][Pmax] starting points of init mode "given" (epg_set_inits), NaN: random
+    int inits_C = 0;
+    std::vector<unsigned char> h_inits_set;   // [K] 1: epg_set_inits covered the site
     CUtensorMap tmap;                   // TMA descriptor of Xb: box 64 columns x 128 rows, 128-byte swizzle
     bool tc_ok = false;                 // tensor-core passes usable (single group, D+1 <= 256)
     int use_tc = 1;                     // option (epg_set_option "use_tc")
@@ -98,7 +102,7 @@ void epg_sites_free(epg_ctx* c) {
     cudaFree(s->xmean); cudaFree(s->gout_w); cudaFree(s->order); cudaFree(s->reinit); cudaFree(s->tstats);
     cudaFree(s->X); cudaFree(s->Xb); cudaFree(s->y); cudaFree(s->row0); cudaFree(s->grp_ptr); cudaFree(s->grp_rows);
     cudaFree(s->chain_mem); cudaFree(s->last_q); cudaFree(s->omega); cudaFree(s->out); cudaFree(s->ld_buf);
-    cudaFree(s->dense); cudaFree(s->dense_ws);
+    cudaFree(s->dense); cudaFree(s->dense_ws); cudaFree(s->inits);
     delete s;
     c->sites = nullptr;
 }
@@ -162,6 +166,7 @@ __device__ __forceinline__ uint4 philox4x32(uint4 ctr, uint2 key) {
     }
     return ctr;
 }
+// purposes: 1 tree uniforms, 2 momenta, 3 random inits, 4 step-size jitter, 5 re-initialisation around the cavity
 __device__ __forceinline__ float u01(uint32_t x) { return ((float)(x >> 8) + 0.5f) * (1.0f / 16777216.0f); }
 __device__ __forceinline__ float rng_uniform(uint2 key, uint32_t& ctr) {
     const uint4 r = philox4x32(make_uint4(ctr++, 0u, 1u, 0u), key);
@@ -203,11 +208,14 @@ enum {
 #define NVEC (V_STACK + 4 * MAXDEPTH_CAP)
 
 enum { PH_START = 0, PH_START_WAIT, PH_SS_WAIT, PH_TREE_WAIT, PH_DONE, PH_DEAD };
+// starting points: the public init modes of epg_sampler_opts (0-3), and the re-initialisation around the cavity
+// of a site marked by epg_reinit_sites
+enum { IM_RANDOM = 0, IM_ZERO = 1, IM_PREV = 2, IM_GIVEN = 3, IM_REINIT = 4 };
 
 struct ChainS {
     int phase, iter, depth, nleaf, sign, n_leap_tr, ss_dir, ss_first, init_tries, restart_ss;
     int carried;                  // the warm-up started from the previous run's adapted metric / step size
-    int init_mode;                // SamplerArgs::init_mode, or 3 (around the cavity mean) for a site marked by epg_reinit_sites
+    int init_mode;                // SamplerArgs::init_mode, or IM_REINIT for a site marked by epg_reinit_sites
     uint32_t rng;
     float eps;
     double V, H0, Vs, lsw, sum_metro, cur_lsw, Vprop;
@@ -216,11 +224,14 @@ struct ChainS {
     int da_count;
     // variance windows
     int win_count, win_next, win_size, w_n;
+    float eps_tr;                 // step size of the current transition: eps (the nominal step size) with jitter applied
     // analytics
     double eps_sum;
     long long n_leap_total;
     int n_div;
 };
+// (the shared-memory plan is built from this size: new fields go into the two 4-byte alignment holes)
+static_assert(sizeof(ChainS) == 184, "ChainS layout");
 // per-level scalars of the tree stack live in shared memory next to ChainS
 struct ChainStack { double lsw[MAXDEPTH_CAP], V[MAXDEPTH_CAP]; };
 
@@ -244,6 +255,11 @@ struct SamplerArgs {
     int iter, warmup, init_mode, max_depth;
     double delta;
     int win_init, win_term, win_base;
+    double gamma, kappa, t0;           // dual averaging (epg_sampler_adapt)
+    float stepsize, jitter, init_r;    // starting nominal step size, step-size jitter, radius of random inits
+    int adapt_engaged;                 // 0: no step-size heuristic, dual averaging or metric windows
+    int thin, n_save;                  // post-warm-up transition m is saved when m % thin == 0; n_save per chain
+    const float* inits;                // init mode "given": [K][C][P] starting points, NaN = random
     const uint32_t* seeds;
     // outputs
     double* draws; int n_draws;     // [K][d][n]
@@ -1067,7 +1083,7 @@ __device__ void begin_ss_trial(const CX& x, ChainS& s) {
 
 template <class CX>
 __device__ void issue_leapfrog(const CX& x, ChainS& s) {
-    leapfrog_begin(x, s.sign * s.eps);
+    leapfrog_begin(x, s.sign * s.eps_tr);
     s.phase = PH_TREE_WAIT;
 }
 
@@ -1084,6 +1100,13 @@ __device__ void begin_subtree(const CX& x, ChainS& s) {
 
 template <class CX>
 __device__ void begin_transition(const CX& x, ChainS& s) {
+    // base_hmc::sample_stepsize: eps = eps_nom (1 + jitter (2u - 1)) from its own stream (counter = transition), so
+    // that jitter 0 draws exactly what a run without jitter draws
+    s.eps_tr = s.eps;
+    if (x.a.jitter > 0.0f) {
+        const uint4 r = philox4x32(make_uint4((uint32_t)s.iter, 0u, 4u, 0u), x.key);
+        s.eps_tr = s.eps * (1.0f + x.a.jitter * (2.0f * u01(r.x) - 1.0f));
+    }
     vcopy(x, V_Q, V_QS);
     vcopy(x, V_G, V_GS);
     __syncwarp();
@@ -1180,13 +1203,14 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
     const float* qs = x.v(V_QS);
     bool restart_ss = false;
     if (s.iter < a.warmup) {
+      if (a.adapt_engaged) {           // (otherwise a warm-up transition is only discarded)
         // ---- dual averaging (stepsize_adaptation::learn_stepsize) ----
         s.da_count += 1;
         const double stat = accept > 1.0 ? 1.0 : accept;
-        const double eta = 1.0 / (s.da_count + 10.0);
+        const double eta = 1.0 / (s.da_count + a.t0);
         s.s_bar = (1.0 - eta) * s.s_bar + eta * (a.delta - stat);
-        const double xx = s.mu - s.s_bar * sqrt((double)s.da_count) / 0.05;
-        const double x_eta = pow((double)s.da_count, -0.75);
+        const double xx = s.mu - s.s_bar * sqrt((double)s.da_count) / a.gamma;
+        const double x_eta = pow((double)s.da_count, -a.kappa);
         s.x_bar = (1.0 - x_eta) * s.x_bar + x_eta * xx;
         s.eps = (float)exp(xx);
         // ---- variance windows (var_adaptation::learn_variance; dense_e: covar_adaptation; unit_e: none) ----
@@ -1247,10 +1271,11 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
             restart_ss = true;
         }
         s.win_count += 1;
-    } else {
-        // ---- store the draw of phi and accumulate split-Rhat sums ----
-        const int t = s.iter - a.warmup;
-        const int per = a.iter - a.warmup;
+      }
+    } else if ((s.iter - a.warmup) % a.thin == 0) {
+        // ---- store the draw of phi (saved draw t of n_save) and accumulate split-Rhat sums ----
+        const int t = (s.iter - a.warmup) / a.thin;
+        const int per = a.n_save;
         double* dst = a.draws + (size_t)k_global_draw_site * a.d * a.n_draws;
         for (int i = x.lane; i < a.d; i += 32) dst[(size_t)i * a.n_draws + c_local * per + t] = (double)qs[i];
         const int half = (t < per / 2) ? 0 : 1;
@@ -1263,7 +1288,13 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
                 rs[i] += dv; rq[i] += dv * dv;
             }
         }
-        s.eps_sum += s.eps;
+        s.eps_sum += s.eps_tr;
+        if (t == per - 1) {
+            // the last saved draw is what init_prev carries over (util.get_last_fit_sample reads the last saved
+            // draw of a fit; with thin > 1 it need not be the final transition)
+            float* lq = a.last_q + (size_t)x.cg * a.P;
+            for (int i = x.lane; i < x.p; i += 32) lq[i] = qs[i];
+        }
         if (a.tstats) {
             // transformed parameters of the Stan programs (m1b.stan:30-36 ...): slot i of q maps to
             // phi_i | alpha_j = [mu_a +] eta_j sigma_a | beta_ji = [mu_b,i +] etb_ji sigma_b,i
@@ -1288,7 +1319,7 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
     }
     __syncwarp();
     s.iter += 1;
-    if (s.iter == a.warmup && a.warmup > 0) {
+    if (s.iter == a.warmup && a.warmup > 0 && a.adapt_engaged) {
         s.eps = (float)exp(s.x_bar);                 // complete_adaptation
         restart_ss = false;
     }
@@ -1299,10 +1330,9 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
         __syncwarp();
     }
     if (s.iter >= a.iter) {
-        float* lq = a.last_q + (size_t)x.cg * a.P;
         float* lm = a.last_minv + (size_t)x.cg * a.P;
         const float* minv = x.v(V_MINV);
-        for (int i = x.lane; i < x.p; i += 32) { lq[i] = qs[i]; lm[i] = minv[i]; }
+        for (int i = x.lane; i < x.p; i += 32) lm[i] = minv[i];
         if (x.lane == 0) { a.last_eps[x.cg] = s.eps; a.last_metric[x.cg] = (float)a.metric; }
         s.phase = PH_DONE;
         return;
@@ -1314,6 +1344,14 @@ __device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global
     } else {
         begin_transition(x, s);
     }
+}
+
+// a given starting point (init mode "given") with an entry to draw at random (NaN)
+template <class CX>
+__device__ bool given_has_random(const CX& x, const float* gq) {
+    float nr = 0.0f;
+    for (int i = x.lane; i < x.p; i += 32) if (isnan(gq[i])) nr = 1.0f;
+    return warp_sum(nr) > 0.0f;
 }
 
 // One step of the per-chain state machine: consume the gradient that was just
@@ -1334,22 +1372,27 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
             vcopy(x, V_QS, V_Q);
             vcopy(x, V_GS, V_G);
             __syncwarp();
+            if (!a.adapt_engaged) { begin_transition(x, s); return; }     // (run_sampler: no step-size heuristic)
             s.ss_first = 1;
             s.restart_ss = 0;
             begin_ss_trial(x, s);
             return;
         }
-        if ((s.init_mode == 0 || s.init_mode == 3) && s.init_tries < 100) { s.init_tries++; s.phase = PH_START; }   // redraw below
+        // redraw a starting point with a random component (Stan: up to 100 attempts); one that is given in full
+        // fails the chain at once
+        const bool redraw = s.init_mode == IM_RANDOM || s.init_mode == IM_REINIT ||
+                            (s.init_mode == IM_GIVEN && given_has_random(x, a.inits + (size_t)x.cg * a.P));
+        if (redraw && s.init_tries < 100) { s.init_tries++; s.phase = PH_START; }   // redraw below
         else { s.phase = PH_DEAD; return; }
     }
     if (s.phase == PH_START) {
         float* q = x.v(V_Q);
-        if (s.init_mode == 2) {
+        if (s.init_mode == IM_PREV) {
             const float* lq = a.last_q + (size_t)x.cg * a.P;
             for (int i = x.lane; i < x.p; i += 32) q[i] = lq[i];
-        } else if (s.init_mode == 1) {
+        } else if (s.init_mode == IM_ZERO) {
             for (int i = x.lane; i < x.p; i += 32) q[i] = 0.0f;
-        } else if (s.init_mode == 3) {
+        } else if (s.init_mode == IM_REINIT) {
             // re-initialisation of a site whose chains did not mix: phi within one conditional cavity standard
             // deviation of the cavity mean, latents in U(-1, 1).  (Late in an EP run the cavity is so tight that
             // Stan's U(-2, 2) starts thousands of standard deviations out and the step size collapses.)
@@ -1360,10 +1403,16 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
                 q[i] = i < x.d ? x.muf()[i] + u * rsqrtf(fmaxf(x.omega[i * x.d + i], 1e-12f)) : u;
             }
         } else {
-            const uint32_t ctr = s.rng++;
+            // Stan's random init U(-init_r, init_r) (default 2), for every entry of a given init that is NaN
+            // (an init given in full draws nothing: it starts the chain's stream where init '0' does)
+            const float* gq = s.init_mode == IM_GIVEN ? a.inits + (size_t)x.cg * a.P : nullptr;
+            const uint32_t ctr = (!gq || given_has_random(x, gq)) ? s.rng++ : 0u;
+            const float rr = a.init_r;
             for (int i = x.lane; i < x.p; i += 32) {
+                const float g = gq ? gq[i] : NAN;
+                if (!isnan(g)) { q[i] = g; continue; }
                 const uint4 r = philox4x32(make_uint4(ctr, (uint32_t)i, 3u, 0u), x.key);
-                q[i] = 4.0f * u01(r.x) - 2.0f;       // Stan's default init: U(-2, 2)
+                q[i] = 2.0f * rr * u01(r.x) - rr;
             }
         }
         __syncwarp();
@@ -1373,7 +1422,7 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
     // ---- consume ----
     double Vnew, kin_leaf = 0.0;
     const bool tree_leaf = s.phase == PH_TREE_WAIT;
-    if (tree_leaf) leaf_fused(x, lp_lik, s.sign * s.eps, Vnew, kin_leaf);
+    if (tree_leaf) leaf_fused(x, lp_lik, s.sign * s.eps_tr, Vnew, kin_leaf);
     else Vnew = finish_gradient(x, lp_lik);
     if (s.phase == PH_SS_WAIT) {
         leapfrog_end(x, s.eps);
@@ -1530,7 +1579,7 @@ __device__ __forceinline__ void load_cavity(const SamplerArgs& a, int k, float* 
 
 // initial state of the site's chains; warp w of a group of nw warps
 __device__ __forceinline__ void init_chains(const SamplerArgs& a, const SiteView& sv, ChainS* cs, int w, int nw, int lane) {
-    const int im = (a.init_mode == 2 && a.reinit && a.reinit[sv.k]) ? 3 : a.init_mode;
+    const int im = (a.init_mode == IM_PREV && a.reinit && a.reinit[sv.k]) ? IM_REINIT : a.init_mode;
     for (int c = w; c < a.C; c += nw) {
         ChainS& s = cs[c];
         const int cg = sv.k * a.C + c;
@@ -1540,9 +1589,11 @@ __device__ __forceinline__ void init_chains(const SamplerArgs& a, const SiteView
         // 90 % of every warm-up crawl at the scale of the tightest cavity direction with saturated trees.
         // A re-initialised site (mode 3) starts from the conditional cavity variances instead.
         // (only from a run of the same metric: a diag_e metric is no starting point for dense_e, nor vice versa)
-        float eps0 = 1.0f;
+        // The step size starts from control 'stepsize' (default 1).  Without adaptation (run_sampler) every chain
+        // runs with that step size and the unit metric throughout.
+        float eps0 = a.stepsize;
         bool carried = false;
-        if (im == 2 && a.carry_adapt && a.last_metric[cg] == (float)a.metric) {
+        if (im == IM_PREV && a.carry_adapt && a.adapt_engaged && a.last_metric[cg] == (float)a.metric) {
             const float e = a.last_eps[cg];
             if (e > 0.0f && isfinite(e)) { eps0 = e; carried = true; }     // (written together with last_minv)
         }
@@ -1560,11 +1611,11 @@ __device__ __forceinline__ void init_chains(const SamplerArgs& a, const SiteView
         // starting inverse metric, element i of the diagonal (unit_e: always 1)
         auto start_minv = [&](int i) -> float {
             float mv = 1.0f;
-            if (a.metric == EPG_METRIC_UNIT) return mv;
+            if (a.metric == EPG_METRIC_UNIT || !a.adapt_engaged) return mv;
             if (carried) {
                 const float v = a.last_minv[(size_t)cg * a.P + i];
                 if (v > 0.0f && isfinite(v)) mv = v;
-            } else if (im == 3 && i < a.d) {
+            } else if (im == IM_REINIT && i < a.d) {
                 const double om = a.cavQ[(size_t)sv.k * a.d * a.d + (size_t)i * a.d + i];
                 if (om > 0.0 && isfinite(om)) mv = (float)(1.0 / om);
             }
@@ -1620,7 +1671,7 @@ __device__ __forceinline__ void chain_phase(const SamplerArgs& a, const SiteView
 __device__ void site_analytics(const SamplerArgs& a, const SiteView& sv, const ChainS* cs, int p, int lane,
                                double clk_chain, double clk_lik, double n_ticks) {
     const int C = a.C;
-    const int per = a.iter - a.warmup;
+    const int per = a.n_save;                    // saved draws per chain
     const int hn = per / 2;
     float worst = 0.0f;
     if (hn >= 2 && C >= 1) {
@@ -2374,26 +2425,82 @@ static void record_plan(epg_site_data* s, const SamplerArgs& a, int kernel, int 
 
 int epg_reserve_draws(epg_ctx* c, int n);
 
+int epg_set_inits(epg_ctx* c, int k0, int k1, int chains, const double* q) {
+    if (!c->sites) return epg_fail_msg(c, "epg_set_inits: no site data (epg_upload_sites)");
+    if (k0 < 0 || k1 > c->K || k0 >= k1 || !q) return epg_fail_msg(c, "epg_set_inits: bad args");
+    if (chains < 1 || chains > 32) return epg_fail_msg(c, "chains must be in 1..32");
+    epg_site_data* s = c->sites;
+    const size_t P = s->Pmax;
+    if (s->inits_C != chains || !s->inits) {
+        // (a new chain count drops the starting points of every site)
+        EPG_CHECK(c, cudaStreamSynchronize(c->stream));
+        cudaFree(s->inits);
+        s->inits = nullptr; s->inits_C = 0;
+        EPG_CHECK(c, cudaMalloc((void**)&s->inits, sizeof(float) * (size_t)c->K * chains * P));
+        s->inits_C = chains;
+        s->h_inits_set.assign((size_t)c->K, 0);
+    }
+    std::vector<float> h((size_t)(k1 - k0) * chains * P);
+    for (size_t i = 0; i < h.size(); ++i) h[i] = (float)q[i];
+    EPG_CHECK(c, cudaMemcpyAsync(s->inits + (size_t)k0 * chains * P, h.data(), sizeof(float) * h.size(),
+                                 cudaMemcpyHostToDevice, c->stream));
+    EPG_CHECK(c, cudaStreamSynchronize(c->stream));           // (h is a local)
+    std::fill(s->h_inits_set.begin() + k0, s->h_inits_set.begin() + k1, (unsigned char)1);
+    return 0;
+}
+
+static const epg_sampler_adapt k_stan_adapt = {1.0, 0.0, 0.05, 0.75, 10.0, 2.0, 1, 75, 50, 25, {0}};
+
 int epg_tilted_sample(epg_ctx* c, int k0, int k1, const uint32_t* seeds, const epg_sampler_opts* o,
                       double* msteps_out, double* mrhat_out, int64_t* n_leapfrog_out, double* seconds) {
+    return epg_tilted_sample_ex(c, k0, k1, seeds, o, nullptr, msteps_out, mrhat_out, n_leapfrog_out, seconds);
+}
+
+int epg_tilted_sample_ex(epg_ctx* c, int k0, int k1, const uint32_t* seeds, const epg_sampler_opts* o,
+                         const epg_sampler_adapt* ad, double* msteps_out, double* mrhat_out,
+                         int64_t* n_leapfrog_out, double* seconds) {
     if (!c->sites) return epg_fail_msg(c, "epg_tilted_sample: no site data (epg_upload_sites)");
     if (k0 < 0 || k1 > c->K || k0 >= k1 || !seeds || !o) return epg_fail_msg(c, "epg_tilted_sample: bad args");
+    if (!ad) ad = &k_stan_adapt;
     if (o->chains < 1 || o->chains > 32) return epg_fail_msg(c, "chains must be in 1..32");
-    if (o->thin != 1) return epg_fail_msg(c, "only thin=1 is supported");
+    if (o->thin < 1) return epg_fail_msg(c, "thin must be >= 1");
     if (o->iter < 1) return epg_fail_msg(c, "iter must be positive");
     if (o->metric < EPG_METRIC_DIAG || o->metric > EPG_METRIC_UNIT)
         return epg_fail_msg(c, "metric must be 0 (diag_e), 1 (dense_e) or 2 (unit_e)");
+    if (o->init_mode < 0 || o->init_mode > 3) return epg_fail_msg(c, "init_mode must be 0, 1, 2 or 3");
+    auto pos = [](double v) { return v > 0.0 && std::isfinite(v); };
+    if (!pos(ad->stepsize) || !((float)ad->stepsize > 0.0f) || !std::isfinite((float)ad->stepsize))
+        return epg_fail_msg(c, "stepsize must be positive and finite");
+    if (!(ad->stepsize_jitter >= 0.0 && ad->stepsize_jitter <= 1.0))
+        return epg_fail_msg(c, "stepsize_jitter must be in [0, 1]");
+    if (!pos(ad->gamma)) return epg_fail_msg(c, "adapt_gamma must be positive");
+    if (!pos(ad->kappa)) return epg_fail_msg(c, "adapt_kappa must be positive");
+    if (!pos(ad->t0)) return epg_fail_msg(c, "adapt_t0 must be positive");
+    if (!pos(ad->init_radius)) return epg_fail_msg(c, "init_radius must be positive and finite");
+    if (ad->engaged != 0 && ad->engaged != 1) return epg_fail_msg(c, "engaged must be 0 or 1");
+    if (ad->init_buffer < 0 || ad->term_buffer < 0) return epg_fail_msg(c, "adaptation buffers must be >= 0");
+    if (ad->window < 1) return epg_fail_msg(c, "adapt_window must be >= 1");
     const int warm = o->warmup < 0 ? o->iter / 2 : o->warmup;
     if (warm >= o->iter) return epg_fail_msg(c, "warmup must be smaller than iter");
     const int C = o->chains, CP = pad_chains(C);
-    const int n = C * (o->iter - warm);
+    const int n_save = (o->iter - warm + o->thin - 1) / o->thin;
+    const int n = C * n_save;
     epg_site_data* s = c->sites;
     if (o->init_mode == 2 && (s->last_C != C || !s->last_q)) return epg_fail_msg(c, "init_prev without previous draws");
+    if (o->init_mode == 3 && (s->inits_C != C || !s->inits ||
+                              !std::all_of(s->h_inits_set.begin() + k0, s->h_inits_set.begin() + k1,
+                                           [](unsigned char f) { return f != 0; })))
+        return epg_fail_msg(c, "init mode 3 (given): epg_set_inits has not set these sites for this chain count");
     if (int rc = epg_reserve_draws(c, n)) return rc;
     SamplerArgs a;
     memset(&a, 0, sizeof(a));
     if (int rc = fill_args(c, a, C, CP, k1 - k0, true)) return rc;
     a.iter = o->iter; a.warmup = warm; a.init_mode = o->init_mode;
+    a.thin = o->thin; a.n_save = n_save;
+    a.gamma = ad->gamma; a.kappa = ad->kappa; a.t0 = ad->t0;
+    a.stepsize = (float)ad->stepsize; a.jitter = (float)ad->stepsize_jitter; a.init_r = (float)ad->init_radius;
+    a.adapt_engaged = ad->engaged;
+    a.inits = o->init_mode == 3 ? s->inits : nullptr;
     a.metric = o->metric;
     if (a.metric == EPG_METRIC_DENSE) {
         // (allocated with the first dense_e run; a larger chain count reallocates them, and the carried state with
@@ -2405,8 +2512,9 @@ int epg_tilted_sample(epg_ctx* c, int k0, int k1, const uint32_t* seeds, const e
     }
     a.max_depth = o->max_treedepth > 0 ? std::min(o->max_treedepth, MAXDEPTH_CAP) : 10;
     a.delta = o->adapt_delta > 0 ? o->adapt_delta : 0.8;
-    // Stan 2.17 windowed_adaptation defaults (75 / 50 / 25) and their rescaling
-    a.win_init = 75; a.win_term = 50; a.win_base = 25;
+    // Stan 2.17 windowed_adaptation::set_window_params: (init buffer, term buffer, window), 75 / 50 / 25 by
+    // default, rescaled to 15 % / 10 % / the rest when they do not fit the warm-up
+    a.win_init = ad->init_buffer; a.win_term = ad->term_buffer; a.win_base = ad->window;
     if (warm >= 20 && a.win_init + a.win_base + a.win_term > warm) {
         a.win_init = (int)(0.15 * warm); a.win_term = (int)(0.1 * warm);
         a.win_base = warm - (a.win_init + a.win_term);

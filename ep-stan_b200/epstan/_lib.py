@@ -31,6 +31,17 @@ class SamplerOpts(C.Structure):
                 ('adapt_delta', C.c_double), ('metric', C.c_int32), ('reserved', C.c_int32 * 7)]
 
 
+class SamplerAdapt(C.Structure):
+    """epg_sampler_adapt: Stan's step-size, adaptation and init-radius settings"""
+    _fields_ = [('stepsize', C.c_double), ('stepsize_jitter', C.c_double), ('gamma', C.c_double),
+                ('kappa', C.c_double), ('t0', C.c_double), ('init_radius', C.c_double), ('engaged', C.c_int32),
+                ('init_buffer', C.c_int32), ('term_buffer', C.c_int32), ('window', C.c_int32),
+                ('reserved', C.c_int32 * 8)]
+
+
+INIT_GIVEN = 3            # init_mode of starting points set by Context.set_inits
+
+
 class EpgError(RuntimeError):
     pass
 
@@ -86,6 +97,10 @@ SYMBOLS = [
                                    _c_int32_p, _c_int32_p]),
     ('epg_tilted_sample', C.c_int, [C.c_void_p, C.c_int, C.c_int, _c_uint32_p, C.POINTER(SamplerOpts),
                                     _c_double_p, _c_double_p, _c_int64_p, _c_double_p]),
+    ('epg_tilted_sample_ex', C.c_int, [C.c_void_p, C.c_int, C.c_int, _c_uint32_p, C.POINTER(SamplerOpts),
+                                       C.POINTER(SamplerAdapt), _c_double_p, _c_double_p, _c_int64_p,
+                                       _c_double_p]),
+    ('epg_set_inits', C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _c_double_p]),
     ('epg_set_option', C.c_int, [C.c_void_p, C.c_char_p, C.c_double]),
     ('epg_num_params', C.c_int, [C.c_void_p, C.c_int]),
     ('epg_logdensity', C.c_int, [C.c_void_p, C.c_int, C.c_int, _c_double_p, _c_double_p, _c_double_p,
@@ -412,24 +427,44 @@ class Context:
             None if jk is None else jk.ctypes.data_as(_c_int32_p)))
 
     def tilted_sample(self, seeds, chains, iter, warmup=None, init_mode=0, k0=0, k1=None,
-                      max_treedepth=10, adapt_delta=0.8, metric='diag_e'):
-        """metric: 'diag_e' (Stan's default), 'dense_e' or 'unit_e'"""
+                      max_treedepth=10, adapt_delta=0.8, metric='diag_e', thin=1, stepsize=1.0,
+                      stepsize_jitter=0.0, adapt_engaged=True, adapt_gamma=0.05, adapt_kappa=0.75, adapt_t0=10.0,
+                      adapt_init_buffer=75, adapt_term_buffer=50, adapt_window=25, init_r=2.0):
+        """metric: 'diag_e' (Stan's default), 'dense_e' or 'unit_e'; init_mode 0 random, 1 zeros, 2 previous
+        last draws, INIT_GIVEN the starting points of set_inits.  The rest are PyStan's `thin`, `init_r` and
+        `control` settings (include/epgpu.h, epg_sampler_adapt); draws per chain: ceil((iter - warmup) / thin)."""
         k1 = self.K if k1 is None else k1
         if metric not in METRICS:
             raise ValueError("metric must be one of %s, not %r" % (sorted(METRICS), metric))
         seeds = np.ascontiguousarray(seeds, dtype=np.uint32)
         assert seeds.size == k1 - k0
-        opts = SamplerOpts(chains=chains, iter=iter, warmup=-1 if warmup is None else warmup, thin=1,
+        opts = SamplerOpts(chains=chains, iter=iter, warmup=-1 if warmup is None else warmup, thin=thin,
                            init_mode=init_mode, max_treedepth=max_treedepth, adapt_delta=adapt_delta,
                            metric=METRICS[metric])
+        adapt = SamplerAdapt(stepsize=stepsize, stepsize_jitter=stepsize_jitter, gamma=adapt_gamma,
+                             kappa=adapt_kappa, t0=adapt_t0, init_radius=init_r, engaged=1 if adapt_engaged else 0,
+                             init_buffer=adapt_init_buffer, term_buffer=adapt_term_buffer, window=adapt_window)
         msteps = np.empty(k1 - k0)
         mrhat = np.empty(k1 - k0)
         nleap = np.empty(k1 - k0, dtype=np.int64)
         secs = C.c_double(0.0)
-        self._ck(self._lib.epg_tilted_sample(
-            self._h, k0, k1, seeds.ctypes.data_as(_c_uint32_p), C.byref(opts), _dp(msteps), _dp(mrhat),
-            nleap.ctypes.data_as(_c_int64_p), C.byref(secs)))
+        self._ck(self._lib.epg_tilted_sample_ex(
+            self._h, k0, k1, seeds.ctypes.data_as(_c_uint32_p), C.byref(opts), C.byref(adapt), _dp(msteps),
+            _dp(mrhat), nleap.ctypes.data_as(_c_int64_p), C.byref(secs)))
         return msteps, mrhat, nleap, secs.value
+
+    def set_inits(self, q, chains, k0=0, k1=None):
+        """starting points of init_mode INIT_GIVEN: q [k1-k0, chains, <= Pmax] (NaN: drawn at random; padded
+        with NaN to Pmax = epg_max_params)"""
+        k1 = self.K if k1 is None else k1
+        q = np.asarray(q, dtype=np.float64)
+        P = int(self._lib.epg_max_params(self._h))
+        if q.ndim != 3 or q.shape[:2] != (k1 - k0, chains) or q.shape[2] > P:
+            raise ValueError("inits of shape %s, expected %s" % (q.shape, (k1 - k0, chains, P)))
+        full = np.full((k1 - k0, chains, P), np.nan)
+        full[:, :, :q.shape[2]] = q
+        q = full
+        self._ck(self._lib.epg_set_inits(self._h, k0, k1, int(chains), _dp(q)))
 
     def set_option(self, name, value):
         self._ck(self._lib.epg_set_option(self._h, name.encode(), float(value)))

@@ -23,6 +23,7 @@ import numpy as np
 
 from . import _lib
 from . import _comm
+from . import util
 from .util import (LinAlgError, BuiltinModel, load_stan, copy_fit_samples,
                    get_last_fit_sample)
 
@@ -61,6 +62,7 @@ class _Shard(object):
         self.ctx, self.k_begin, self.k_end, self.K, self.comm = ctx, k_begin, k_end, K, comm
         self.n_local = k_end - k_begin
         self.sites_uploaded = False
+        self.inits_set = set()          # local sites whose dict / list / function `init` is on the device
 
     def local(self, k):
         if not (self.k_begin <= k < self.k_end):
@@ -100,11 +102,20 @@ class Worker(object):
         'warmup'          : None,
         'thin'            : 1,
         'init'            : 'random',
+        # extension (PyStan's own `sampling` keyword, which the reference never sets): radius of the random
+        # inits U(-init_r, init_r); None = Stan's 2 (and not passed to a caller-supplied sampler)
+        'init_r'          : None,
         # extension (PyStan's own `sampling` keyword, which the reference never sets): NUTS controls of the
-        # built-in sampler, {'max_treedepth': int, 'adapt_delta': float, 'metric': 'diag_e' | 'dense_e' |
-        # 'unit_e'}; None = Stan's defaults (10, 0.8, 'diag_e')
+        # built-in sampler, any of CONTROL_KEYS; None = Stan's defaults
         'control'         : None
     }
+
+    # PyStan 2.17's `control` keys (Stan's defaults): max_treedepth 10, adapt_delta 0.8, metric 'diag_e'
+    # ('dense_e', 'unit_e'), stepsize 1, stepsize_jitter 0, adapt_engaged True, adapt_gamma 0.05, adapt_kappa 0.75,
+    # adapt_t0 10, adapt_init_buffer 75, adapt_term_buffer 50, adapt_window 25 (include/epgpu.h, epg_sampler_adapt)
+    CONTROL_KEYS = ('max_treedepth', 'adapt_delta', 'metric', 'stepsize', 'stepsize_jitter', 'adapt_engaged',
+                    'adapt_gamma', 'adapt_kappa', 'adapt_t0', 'adapt_init_buffer', 'adapt_term_buffer',
+                    'adapt_window')
 
     PREC_ESTIM_OPTIONS = ('sample', 'olse')
 
@@ -156,24 +167,10 @@ class Worker(object):
         self.last_n_leapfrog = 0
         self.saved_samples = None
 
-        if self.builtin:
-            # the built-in sampler keeps every post-warm-up draw and starts from 'random', '0' or the
-            # previous draws: anything else would silently change the number of draws / the estimator
-            if self.stan_params['thin'] != 1:
-                raise ValueError("built-in sampler supports thin=1 only (got thin={})".format(
-                    self.stan_params['thin']))
-            if self.stan_params['init'] not in ('random', '0', 0):
-                raise ValueError("built-in sampler supports init 'random' or '0' only")
-            ctl = self.stan_params['control']
-            if ctl is not None and (not isinstance(ctl, dict) or
-                                    set(ctl) - {'max_treedepth', 'adapt_delta', 'metric'}):
-                raise ValueError("built-in sampler: `control` may hold 'max_treedepth', 'adapt_delta' and "
-                                 "'metric' only")
-            if ctl is not None and ctl.get('metric', 'diag_e') not in _lib.METRICS:
-                raise ValueError("built-in sampler: control['metric'] must be one of {} (got {!r})".format(
-                    sorted(_lib.METRICS), ctl['metric']))
         self.init_prev = options['init_prev']
         self.adapt_prev = bool(options['adapt_prev'])
+        if self.builtin:
+            self._check_sampler_args()
         self.init_orig = self.stan_params['init']
         if self.init_prev and not isinstance(self.init_orig, str):
             raise ValueError("Arg. `init` has to be a string if `init_prev` is True")
@@ -195,10 +192,75 @@ class Worker(object):
         self._shard = shard
 
     # -- helpers -------------------------------------------------------------
+    def _check_sampler_args(self):
+        """ValueError for a sampling argument the built-in sampler cannot honour as PyStan would"""
+        sp = self.stan_params
+
+        def is_int(v):
+            return isinstance(v, (int, np.integer)) and not isinstance(v, bool)
+
+        def is_pos(v):
+            return isinstance(v, (int, float, np.integer, np.floating)) and not isinstance(v, bool) and \
+                np.isfinite(v) and v > 0
+        if not (is_int(sp['thin']) and sp['thin'] >= 1):
+            raise ValueError("`thin` must be an integer >= 1 (got {!r})".format(sp['thin']))
+        init = sp['init']
+        if isinstance(init, str):
+            if init not in ('random', '0'):
+                raise ValueError("`init` must be 'random', '0', a dict, a list of dicts or a function "
+                                 "(got {!r})".format(init))
+        elif isinstance(init, (list, tuple)):
+            if len(init) != sp['chains'] or not all(isinstance(v, dict) for v in init):
+                raise ValueError("`init` as a list needs one dict per chain ({})".format(sp['chains']))
+        elif not (isinstance(init, dict) or callable(init) or (is_int(init) and init == 0)):
+            raise ValueError("`init` must be 'random', '0', a dict, a list of dicts or a function")
+        if sp['init_r'] is not None and not is_pos(sp['init_r']):
+            raise ValueError("`init_r` must be positive (got {!r})".format(sp['init_r']))
+        ctl = sp['control']
+        if ctl is None:
+            return
+        if not isinstance(ctl, dict) or set(ctl) - set(self.CONTROL_KEYS):
+            raise ValueError("built-in sampler: `control` may hold {} only".format(', '.join(self.CONTROL_KEYS)))
+        if ctl.get('metric', 'diag_e') not in _lib.METRICS:
+            raise ValueError("built-in sampler: control['metric'] must be one of {} (got {!r})".format(
+                sorted(_lib.METRICS), ctl['metric']))
+        for key in ('stepsize', 'adapt_gamma', 'adapt_kappa', 'adapt_t0'):
+            if key in ctl and not is_pos(ctl[key]):
+                raise ValueError("control['{}'] must be positive and finite (got {!r})".format(key, ctl[key]))
+        if 'stepsize_jitter' in ctl:
+            j = ctl['stepsize_jitter']
+            if not (isinstance(j, (int, float, np.integer, np.floating)) and not isinstance(j, bool)
+                    and 0 <= j <= 1):
+                raise ValueError("control['stepsize_jitter'] must be in [0, 1] (got {!r})".format(j))
+        if 'adapt_engaged' in ctl and not (isinstance(ctl['adapt_engaged'], (bool, np.bool_)) or
+                                           (is_int(ctl['adapt_engaged']) and ctl['adapt_engaged'] in (0, 1))):
+            raise ValueError("control['adapt_engaged'] must be a bool (got {!r})".format(ctl['adapt_engaged']))
+        for key, lo in (('adapt_init_buffer', 0), ('adapt_term_buffer', 0), ('adapt_window', 1)):
+            if key in ctl and not (is_int(ctl[key]) and ctl[key] >= lo):
+                raise ValueError("control['{}'] must be an integer >= {} (got {!r})".format(key, lo, ctl[key]))
+        if 'stepsize' in ctl and self.init_prev and self.adapt_prev and ctl.get('adapt_engaged', True):
+            # every run after the first starts from the carried step size: the value would apply once only
+            raise ValueError("control['stepsize'] with init_prev and adapt_prev (the defaults) would set the "
+                             "first EP iteration's step size only: pass adapt_prev=False")
+
+    def _sampler_kw(self):
+        """keyword arguments of Context.tilted_sample beyond the run's shape"""
+        sp = self.stan_params
+        kw = dict(sp['control'] or {})
+        kw['thin'] = int(sp['thin'])
+        if sp['init_r'] is not None:
+            kw['init_r'] = float(sp['init_r'])
+        return kw
+
+    def _site_layout(self):
+        """(family, D, J) of the site: what util.init_values needs"""
+        J = 1 if self.stan_model.single_group else int(self.A['J'])
+        return (self.stan_model.family, self.X.shape[1], J)
+
     def _nsamp(self):
         sp = self.stan_params
         warm = sp['iter'] // 2 if sp['warmup'] is None else sp['warmup']
-        return sp['chains'] * (sp['iter'] - warm)
+        return sp['chains'] * (-(-(sp['iter'] - warm) // sp['thin']))
 
     def _mode_now(self):
         """prec_estim to use this iteration (method.py:413,436-437)."""
@@ -210,19 +272,25 @@ class Worker(object):
         if self.init_prev and self._have_prev:
             return 2
         init = self.stan_params['init']
-        if init == 'random':
-            return 0
-        if init in ('0', 0):
+        if isinstance(init, str):
+            if init == 'random':
+                return 0
+            if init == '0':
+                return 1
+        elif isinstance(init, (dict, list, tuple)) or callable(init):
+            return _lib.INIT_GIVEN
+        elif init == 0:
             return 1
-        raise ValueError("built-in sampler supports init 'random' or '0' only")
+        raise ValueError("`init` must be 'random', '0', a dict, a list of dicts or a function")
 
     def _host_sample(self, seed_stan, save_samples):
         """Draws from a caller-supplied PyStan-style sampler object
         (the reference's in-process branch, method.py:369-397)."""
         t0 = time.perf_counter()
         params = dict(self.stan_params, seed=seed_stan, refresh=-1)
-        if params.get('control') is None:
-            params.pop('control', None)            # (the reference never passes it)
+        for kw in ('control', 'init_r'):
+            if params.get(kw) is None:
+                params.pop(kw, None)               # (the reference never passes them)
         fit = self.stan_model.sampling(data=self.data, **params)
         self.last_time = time.perf_counter() - t0
         self.last_msteps = float(np.mean([np.mean(p['stepsize__']) for p in fit.get_sampler_params()]))
@@ -273,9 +341,11 @@ class Worker(object):
         ctx.upload(_lib.CAVM, np.ascontiguousarray(self.vec), kl, kl + 1)
         if self.builtin:
             sp = self.stan_params
+            mode = self._init_mode()
+            if mode == _lib.INIT_GIVEN:
+                _upload_inits(sh, [self])
             msteps, mrhat, nleap, secs = ctx.tilted_sample(
-                [seed_stan], sp['chains'], sp['iter'], sp['warmup'], self._init_mode(), kl, kl + 1,
-                **(sp['control'] or {}))
+                [seed_stan], sp['chains'], sp['iter'], sp['warmup'], mode, kl, kl + 1, **self._sampler_kw())
             self.last_time, self.last_msteps, self.last_mrhat = secs, float(msteps[0]), float(mrhat[0])
             self.last_n_leapfrog = int(nleap[0])
             self._have_prev = True
@@ -325,6 +395,19 @@ def _upload_site_block(shard, model, workers):
     shard.ctx.upload_sites(model.model_id, D, k_lim, X, y, j_ind, Jk)
     shard.ctx.set_option('carry_adapt', 1 if workers[0].adapt_prev else 0)
     shard.sites_uploaded = True
+    shard.inits_set = set()
+
+
+def _upload_inits(shard, workers):
+    """Starting points of a dict / list / function `init` for a contiguous block of local sites, once per
+    context (a function is called once per chain here, not once per EP iteration)."""
+    kls = [shard.local(w.index) for w in workers]
+    if all(k in shard.inits_set for k in kls):
+        return
+    sp = workers[0].stan_params
+    q = util.init_values(sp['init'], sp['chains'], [w._site_layout() for w in workers])
+    shard.ctx.set_inits(q, sp['chains'], kls[0], kls[-1] + 1)
+    shard.inits_set.update(kls)
 
 
 class Master(object):
@@ -790,8 +873,11 @@ class Master(object):
             modes = set(w._init_mode() for w in workers)
             if len(modes) != 1:
                 raise RuntimeError("sites disagree on the initialisation mode")
+            mode = modes.pop()
+            if mode == _lib.INIT_GIVEN:
+                _upload_inits(sh, workers)
             msteps, mrhat, nleap, secs = ctx.tilted_sample(
-                stan_seeds, sp['chains'], sp['iter'], sp['warmup'], modes.pop(), **(sp['control'] or {}))
+                stan_seeds, sp['chains'], sp['iter'], sp['warmup'], mode, **workers[0]._sampler_kw())
             for i, w in enumerate(workers):
                 w.last_time, w.last_msteps, w.last_mrhat = secs, float(msteps[i]), float(mrhat[i])
                 w.last_n_leapfrog = int(nleap[i])

@@ -222,6 +222,71 @@ def load_stan(filename, overwrite=False):
     return BuiltinModel(os.path.basename(filename))
 
 
+def _init_dict(init, c):
+    """the init dict of chain c: PyStan calls a function as init(chain_id=c) if it takes that argument"""
+    if callable(init):
+        import inspect
+        try:
+            params = inspect.signature(init).parameters
+        except (TypeError, ValueError):
+            params = {}
+        return init(chain_id=c) if 'chain_id' in params else init()
+    if isinstance(init, dict):
+        return init
+    return init[c]
+
+
+def init_values(init, chains, sites, Pmax=None):
+    """Starting points of the built-in sampler for PyStan's ``init`` = dict, list of ``chains`` dicts or a
+    function returning a dict, as the array ``[len(sites)][chains][Pmax]`` that ``Context.set_inits`` takes.
+
+    ``sites`` holds ``(family, D, J)`` per site (family: 'm1b' ... 'm5b'); Pmax None: the largest number of
+    parameters of these sites (Context.set_inits pads to its own).  A site's row is laid out as the
+    sampler's parameter vector ``q = [phi (d) | eta (J) | etb]`` with ``etb`` (J, D) row-major for m3b, m4b and
+    m5b, (D,) for m2b and absent for m1b; a single-group site (J = 1) also takes ``eta`` as a scalar and
+    ``etb`` as (D,).  A parameter missing from the dict is NaN (drawn at random by the sampler), unknown names
+    are ignored as Stan ignores them, and a value of the wrong shape raises ``ValueError``.
+    """
+    if isinstance(init, (list, tuple)):
+        if len(init) != chains:
+            raise ValueError("init: a list of {} dicts for {} chains".format(len(init), chains))
+    elif not (isinstance(init, dict) or callable(init)):
+        raise ValueError("init must be 'random', '0', a dict, a list of dicts or a function returning a dict")
+    dicts = [_init_dict(init, c) for c in range(chains)]
+    for c, dc in enumerate(dicts):
+        if not isinstance(dc, dict):
+            raise ValueError("init of chain {} is not a dict".format(c))
+    layouts = []
+    for family, D, J in sites:
+        d = {'m1b': D + 1, 'm2b': 2, 'm3b': D + 1, 'm4b': 2 * D + 2, 'm5b': 2 * D + 2}[family]
+        layout = [('phi', (d,)), ('eta', (J,))]
+        if family == 'm2b':
+            layout.append(('etb', (D,)))
+        elif family != 'm1b':
+            layout.append(('etb', (J, D)))
+        layouts.append(layout)
+    n_par = [sum(int(np.prod(shp)) for _, shp in layout) for layout in layouts]
+    if Pmax is None:
+        Pmax = max(n_par)
+    elif max(n_par) > Pmax:
+        raise ValueError("init: a site has more parameters ({}) than Pmax = {}".format(max(n_par), Pmax))
+    out = np.full((len(sites), chains, Pmax), np.nan)
+    for k, ((family, D, J), layout) in enumerate(zip(sites, layouts)):
+        for c, dc in enumerate(dicts):
+            off = 0
+            for name, shp in layout:
+                size = int(np.prod(shp))
+                if name in dc:
+                    v = np.asarray(dc[name], dtype=np.float64)
+                    grouped = name == 'eta' or (name == 'etb' and family != 'm2b')
+                    if v.shape != shp and not (J == 1 and grouped and v.shape == shp[1:]):
+                        raise ValueError("init: site {}, parameter '{}': shape {}, expected {}"
+                                         .format(k, name, v.shape, shp))
+                    out[k, c, off:off + size] = v.ravel()
+                off += size
+    return out
+
+
 def distribute_groups(J, K, Nj):
     """Distribute J groups to K sites (reference util.py:540-639).
 

@@ -216,8 +216,11 @@ typedef struct epg_sampler_opts {
     int32_t chains;        /* method.py:155 */
     int32_t iter;          /* method.py:156 */
     int32_t warmup;        /* <0: iter/2  (method.py:567-569) */
-    int32_t thin;          /* only 1 is supported (fit.py:304) */
-    int32_t init_mode;     /* 0: 'random' U(-2,2); 1: zeros; 2: previous last draws (init_prev, method.py:404-406) */
+    int32_t thin;          /* >= 1: post-warm-up transition m (0-based) is saved when m % thin == 0, i.e.
+                              ceil((iter - warmup) / thin) draws per chain (Stan's generate_transitions); the
+                              chain itself, its transitions and random numbers, do not depend on it (fit.py:304) */
+    int32_t init_mode;     /* 0: 'random' U(-init_radius, init_radius); 1: zeros; 2: previous last draws (init_prev,
+                              method.py:404-406); 3: given by epg_set_inits (PyStan init=dict / list / function) */
     int32_t max_treedepth; /* Stan default 10 */
     double adapt_delta;    /* Stan default 0.8 */
     int32_t metric;        /* EPG_METRIC_*; 0 (diag_e) is Stan's default.  Other values: the call fails (< 0) */
@@ -237,6 +240,39 @@ typedef struct epg_sampler_opts {
  * the warm-up starts from Sigma = I and step size 1. */
 enum epg_metric { EPG_METRIC_DIAG = 0, EPG_METRIC_DENSE = 1, EPG_METRIC_UNIT = 2 };
 
+/* Stan 2.17's remaining NUTS settings (PyStan `control`, `init_r`); epg_tilted_sample_ex with adapt == NULL, and
+ * epg_tilted_sample, use the defaults in brackets.  Fill in every field: an out-of-range value fails the call (< 0).
+ *   stepsize         starting nominal step size [1]; the step-size heuristic and dual averaging start from it
+ *                    (mu = log(10 stepsize)).  A chain that carries its adaptation (init_mode 2, carry_adapt) starts
+ *                    from its carried step size instead.  > 0, finite
+ *   stepsize_jitter  j in [0, 1] [0]: every transition (warm-up and sampling) uses eps = eps_nom (1 + j (2u - 1)),
+ *                    u ~ U(0, 1) (base_hmc::sample_stepsize); adaptation works on eps_nom, the mean step size
+ *                    (msteps_out) averages the eps of the saved transitions, like Stan's stepsize__, and the step
+ *                    size carried over is eps_nom
+ *   gamma, kappa, t0 dual-averaging constants of stepsize_adaptation [0.05, 0.75, 10], each > 0
+ *   init_radius      r > 0 [2]: random inits (init_mode 0, and the NaN entries of init_mode 3) are U(-r, r)
+ *   engaged          1 [1]: adaptive NUTS (run_adaptive_sampler); 0: run_sampler -- no step-size heuristic, no
+ *                    dual averaging, no metric windows: eps_nom = stepsize and the inverse metric is the identity
+ *                    throughout, for every metric, init mode and carried state; warm-up transitions still run and
+ *                    are discarded
+ *   init_buffer, term_buffer, window   windowed_adaptation [75, 50, 25]: buffers >= 0, window >= 1.  No windows
+ *                    below 20 warm-up iterations; when init_buffer + window + term_buffer exceeds the warm-up they
+ *                    become 15 % / 10 % / the rest of it (set_window_params); window ends by compute_next_window
+ * (C99) */
+typedef struct epg_sampler_adapt {
+    double stepsize;
+    double stepsize_jitter;
+    double gamma;
+    double kappa;
+    double t0;
+    double init_radius;
+    int32_t engaged;
+    int32_t init_buffer;
+    int32_t term_buffer;
+    int32_t window;
+    int32_t reserved[8];
+} epg_sampler_adapt;
+
 /* Runs adaptive NUTS for sites [k0,k1) x chains on their tilted densities
  * (cavity from EPG_CAVQ/EPG_CAVM x site likelihood), leaves the post-warm-up
  * draws of phi in the device draw buffer ([d][n] per site, chain-major rows,
@@ -248,6 +284,19 @@ enum epg_metric { EPG_METRIC_DIAG = 0, EPG_METRIC_DENSE = 1, EPG_METRIC_UNIT = 2
 int epg_tilted_sample(epg_ctx* ctx, int k0, int k1, const uint32_t* seeds,
                       const epg_sampler_opts* opts, double* msteps_out, double* mrhat_out,
                       int64_t* n_leapfrog_out, double* seconds);
+/* the same with the settings of `adapt` (NULL: Stan's defaults, as epg_tilted_sample) */
+int epg_tilted_sample_ex(epg_ctx* ctx, int k0, int k1, const uint32_t* seeds,
+                         const epg_sampler_opts* opts, const epg_sampler_adapt* adapt, double* msteps_out,
+                         double* mrhat_out, int64_t* n_leapfrog_out, double* seconds);
+
+/* Starting points of init_mode 3 (PyStan init = dict, list of dicts or function): q [k1-k0][chains][Pmax]
+ * (Pmax = epg_max_params) in the layout q = [phi (d) | eta (J) | etb] of epg_get_param_stats.  A NaN entry is
+ * drawn U(-init_radius, init_radius) as init_mode 0 draws it; entries beyond a site's epg_num_params are
+ * ignored.  A chain whose start has a random entry redraws up to 100 times when its density is not finite; one
+ * given in full fails its site at once, as Stan fails such a user init.  The values stay until the next
+ * epg_set_inits or epg_upload_sites; a call with another chain count drops those of every site.  An init_mode 3
+ * run fails unless every one of its sites was set for its chain count. */
+int epg_set_inits(epg_ctx* ctx, int k0, int k1, int chains, const double* q);
 
 /* Marks local sites whose chains the next epg_tilted_sample with init_mode 2 starts afresh -- phi within one
  * conditional cavity standard deviation of the cavity mean, the site-local latents in U(-1,1) -- instead of
