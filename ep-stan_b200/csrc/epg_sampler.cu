@@ -94,6 +94,15 @@ struct epg_site_data {
     double* dense_ws = nullptr;         // dense_e window-end factorisation scratch [K*C][P][P]
     size_t dense_ws_bytes = 0;
     int32_t plan[EPG_PLAN_FIELDS] = {}; // launch plan of the last epg_tilted_sample / epg_logdensity (epg_last_plan)
+    // HMC diagnostics (epg_get_hmc_diag, epg_get_sampler_params)
+    void* hmc = nullptr;                // HmcChain [K*hmc_C]
+    int hmc_C = 0;
+    std::vector<unsigned char> h_hmc_ok;      // [K] 1: the site's most recent run wrote its diagnostics
+    int sampler_params = 0;             // option "sampler_params": record every transition
+    double* rec = nullptr;              // [K][hmc_C][rec_n][HMC_REC]
+    size_t rec_bytes = 0;
+    int rec_iter = 0, rec_warmup = 0, rec_thin = 0, rec_n = 0, rec_nw = 0;   // shape of the records
+    std::vector<unsigned char> h_rec_ok;      // [K] 1: the site's most recent run recorded
 };
 
 void epg_sites_free(epg_ctx* c) {
@@ -102,7 +111,7 @@ void epg_sites_free(epg_ctx* c) {
     cudaFree(s->xmean); cudaFree(s->gout_w); cudaFree(s->order); cudaFree(s->reinit); cudaFree(s->tstats);
     cudaFree(s->X); cudaFree(s->Xb); cudaFree(s->y); cudaFree(s->row0); cudaFree(s->grp_ptr); cudaFree(s->grp_rows);
     cudaFree(s->chain_mem); cudaFree(s->last_q); cudaFree(s->omega); cudaFree(s->out); cudaFree(s->ld_buf);
-    cudaFree(s->dense); cudaFree(s->dense_ws); cudaFree(s->inits);
+    cudaFree(s->dense); cudaFree(s->dense_ws); cudaFree(s->inits); cudaFree(s->hmc); cudaFree(s->rec);
     delete s;
     c->sites = nullptr;
 }
@@ -234,6 +243,16 @@ struct ChainS {
 static_assert(sizeof(ChainS) == 184, "ChainS layout");
 // per-level scalars of the tree stack live in shared memory next to ChainS
 struct ChainStack { double lsw[MAXDEPTH_CAP], V[MAXDEPTH_CAP]; };
+// HMC diagnostics of a chain, in global memory (the shared-memory plan has no room for them): the Hamiltonian
+// H(q, p) of the current sample and of the proposal pending at each tree-stack level (energy__ is H of the
+// selected sample), and the summary of the saved post-warm-up transitions.  Written by lane 0.
+struct HmcChain {
+    double Hs, Hstk[MAXDEPTH_CAP];
+    double e0, se, see, sdd, eprev;     // energies: the first saved one, sums of E - e0, of (E - e0)^2, of
+                                        // (E_t - E_t-1)^2, the previous one
+    double n_saved, n_div, n_maxd, ebfmi;   // the EPG_DIAG_FIELDS of epg_get_hmc_diag, in order
+};
+#define HMC_REC 6                       // values of a per-transition record (PyStan's get_sampler_params order)
 
 struct SamplerArgs {
     // site data
@@ -265,6 +284,9 @@ struct SamplerArgs {
     double* draws; int n_draws;     // [K][d][n]
     double* tstats;                 // [K][2][P] or nullptr (see epg_site_data)
     double* out;                    // [K][8]: mean eps, max rhat, n_leapfrog, n_divergent, clk chain, clk lik, ticks, -
+    HmcChain* hmc;                  // [K*C] HMC diagnostics (always)
+    double* rec;                    // [K][C][n_rec][HMC_REC] per-transition records (option "sampler_params"), or nullptr
+    int n_rec, n_rec_warm;          // records per chain: ceil(warmup / thin) warm-up ones, then the n_save saved ones
     int k0;
     // shared-memory plan
     int R, resident, slices, NC, combos;
@@ -1113,6 +1135,7 @@ __device__ void begin_transition(const CX& x, ChainS& s) {
     sample_momentum(x, s);
     s.V = s.Vs;
     s.H0 = s.Vs + kinetic(x, x.v(V_P));
+    if (x.lane == 0) x.a.hmc[x.cg].Hs = s.H0;           // the sample starts as the initial point
     vcopy(x, V_QM, V_Q); vcopy(x, V_PM, V_P); vcopy(x, V_GM, V_G);
     vcopy(x, V_QP, V_Q); vcopy(x, V_PP, V_P); vcopy(x, V_GP, V_G);
     vcopy(x, V_RHO, V_P);
@@ -1193,12 +1216,45 @@ __device__ void dense_window_end(const CX& x, int n) {
     __syncwarp();
 }
 
+// HMC diagnostics of the transition that ends (lane 0), with Stan 2.17's definitions (base_nuts::transition):
+// the record of every transition Stan saves with save_warmup (warm-up or post-warm-up transition m with
+// m % thin == 0), and over the saved post-warm-up ones the divergences, the transitions at max_treedepth and the
+// energy sums of E-BFMI = sum (E_t - E_t-1)^2 / sum (E_t - mean E)^2 (PyStan's check_energy), shifted by the
+// first saved energy
+template <class CX>
+__device__ void hmc_diagnostics(const CX& x, const ChainS& s, double accept, bool divergent) {
+    const SamplerArgs& a = x.a;
+    const bool warm = s.iter < a.warmup;
+    const int m = warm ? s.iter : s.iter - a.warmup;
+    if (x.lane != 0 || m % a.thin != 0) return;
+    HmcChain& h = a.hmc[x.cg];
+    const double E = h.Hs;
+    const int t = m / a.thin;
+    if (a.rec) {
+        double* r = a.rec + ((size_t)x.cg * a.n_rec + (warm ? 0 : a.n_rec_warm) + t) * HMC_REC;
+        r[0] = accept; r[1] = (double)s.eps_tr; r[2] = (double)s.depth; r[3] = (double)s.n_leap_tr;
+        r[4] = divergent ? 1.0 : 0.0; r[5] = E;
+    }
+    if (warm) return;
+    if (t == 0) { h.e0 = E; h.eprev = E; }
+    const double dv = E - h.e0, de = E - h.eprev;
+    h.se += dv; h.see += dv * dv; h.sdd += de * de; h.eprev = E;
+    h.n_saved += 1.0;
+    if (divergent) h.n_div += 1.0;
+    if (s.depth >= a.max_depth) h.n_maxd += 1.0;
+    if (t == a.n_save - 1) {
+        const double var = h.see - h.se * h.se / h.n_saved;
+        h.ebfmi = (h.n_saved >= 2.0 && var > 0.0) ? h.sdd / var : NAN;
+    }
+}
+
 // bookkeeping at the end of a transition; returns with the next request issued
 // (or the chain finished)
 template <class CX>
-__device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global_draw_site) {
+__device__ void end_transition(const CX& x, ChainS& s, int c_local, int k_global_draw_site, bool divergent) {
     const SamplerArgs& a = x.a;
     const double accept = s.n_leap_tr > 0 ? s.sum_metro / (double)s.n_leap_tr : 0.0;
+    hmc_diagnostics(x, s, accept, divergent);
     s.n_leap_total += s.n_leap_tr;
     const float* qs = x.v(V_QS);
     bool restart_ss = false;
@@ -1460,13 +1516,19 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
     s.sum_metro += (dH > 0.0) ? 1.0 : (double)__expf((float)dH);
     if (-dH > 1000.0) {                 // divergent: the subtree is discarded
         s.n_div += 1;
-        end_transition(x, s, c_local, site_draw);
+        end_transition(x, s, c_local, site_draw, true);
         return;
     }
     // (leaf node vectors -- rho = p, p_sharp(left) = M^-1 p, proposal = this point -- were
     //  written by leaf_fused)
     s.cur_lsw = dH;
     s.Vprop = Vnew;
+    // Hamiltonian of the proposal, beside Vprop (only lane 0 keeps it: it feeds the HMC diagnostics alone): this
+    // leaf's, or that of the highest stack level whose pending proposal wins a merge below, loaded once after the
+    // merges and stored after the next stretch of work
+    HmcChain& hm = a.hmc[x.cg];
+    double hprop = h;
+    int hsrc = -1;
     int l = 0;
     while ((s.nleaf >> l) & 1) {
         // merge the pending left sibling at level l with the node just completed
@@ -1502,15 +1564,17 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
             vcopy(x, V_QPROP, base + 2);
             vcopy(x, V_GPROP, base + 3);
             s.Vprop = x.stk->V[l];
+            hsrc = l;
         }
         __syncwarp();
         s.cur_lsw = lsw_sub;
         if (!(d1 > 0.0f && d2 > 0.0f)) {        // U-turn inside the new subtree: discard it
-            end_transition(x, s, c_local, site_draw);
+            end_transition(x, s, c_local, site_draw, false);
             return;
         }
         ++l;
     }
+    if (x.lane == 0 && hsrc >= 0) hprop = hm.Hstk[hsrc];
     if (l < s.depth) {
         const int base = V_STACK + 4 * l;
         {
@@ -1524,6 +1588,7 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
         __syncwarp();
         s.nleaf += 1;
         issue_leapfrog(x, s);
+        if (x.lane == 0) hm.Hstk[l] = hprop;
         return;
     }
     // ---- the subtree of 2^depth leaves is complete and valid ----
@@ -1558,8 +1623,9 @@ __device__ void chain_step(const CX& x, ChainS& s, double lp_lik, int c_local, i
         d1 = warp_sum(d1); d2 = warp_sum(d2);
         __syncwarp();
     }
+    if (take && x.lane == 0) hm.Hs = hprop;
     if (!(d1 > 0.0f && d2 > 0.0f) || s.depth >= a.max_depth) {
-        end_transition(x, s, c_local, site_draw);
+        end_transition(x, s, c_local, site_draw, false);
         return;
     }
     begin_subtree(x, s);
@@ -1607,6 +1673,9 @@ __device__ __forceinline__ void init_chains(const SamplerArgs& a, const SiteView
             s.rng = 0;
             s.win_next = a.win_init + a.win_base - 1;
             s.win_size = a.win_base;
+            HmcChain& h = a.hmc[cg];
+            memset(&h, 0, sizeof(HmcChain));
+            h.ebfmi = NAN;
         }
         // starting inverse metric, element i of the diagonal (unit_e: always 1)
         auto start_minv = [&](int i) -> float {
@@ -1719,6 +1788,11 @@ __device__ void site_analytics(const SamplerArgs& a, const SiteView& sv, const C
         for (int e = lane; e < a.d * per; e += 32) {
             const int i = e / per, t = e - i * per;
             dst[(size_t)i * a.n_draws + c * per + t] = NAN;
+        }
+        // nor sampler-parameter records (epg_get_sampler_params then returns NaN for it, not stale records)
+        if (a.rec) {
+            double* r = a.rec + (size_t)(sv.k * C + c) * a.n_rec * HMC_REC;
+            for (int e = lane; e < a.n_rec * HMC_REC; e += 32) r[e] = NAN;
         }
     }
     if (a.tstats) {
@@ -2315,6 +2389,11 @@ int epg_set_option(epg_ctx* c, const char* name, double value) {
         c->sites->param_stats = value != 0.0;
         return 0;
     }
+    if (strcmp(name, "sampler_params") == 0) {
+        if (!c->sites) return epg_fail_msg(c, "epg_set_option(sampler_params): upload the sites first");
+        c->sites->sampler_params = value != 0.0;
+        return 0;
+    }
     if (strcmp(name, "carry_adapt") == 0) {
         if (!c->sites) return epg_fail_msg(c, "epg_set_option(carry_adapt): upload the sites first");
         c->sites->carry_adapt = value != 0.0;
@@ -2519,6 +2598,31 @@ int epg_tilted_sample_ex(epg_ctx* c, int k0, int k1, const uint32_t* seeds, cons
         a.win_init = (int)(0.15 * warm); a.win_term = (int)(0.1 * warm);
         a.win_base = warm - (a.win_init + a.win_term);
     }
+    // HMC diagnostics: one block per chain of this chain count (another count drops the diagnostics and records
+    // of every site, as epg_set_inits drops its starting points); records of this shape (another shape drops
+    // those of every other site)
+    if (s->hmc_C != C || !s->hmc) {
+        EPG_CHECK(c, cudaStreamSynchronize(c->stream));
+        cudaFree(s->hmc);
+        s->hmc = nullptr; s->hmc_C = 0;
+        EPG_CHECK(c, cudaMalloc(&s->hmc, sizeof(HmcChain) * (size_t)c->K * C));
+        s->hmc_C = C;
+        s->h_hmc_ok.assign((size_t)c->K, 0);
+        s->h_rec_ok.assign((size_t)c->K, 0);
+    }
+    a.hmc = static_cast<HmcChain*>(s->hmc);
+    const int n_rec_warm = (warm + o->thin - 1) / o->thin;
+    if (s->sampler_params) {
+        if (s->rec_iter != o->iter || s->rec_warmup != warm || s->rec_thin != o->thin) {
+            std::fill(s->h_rec_ok.begin(), s->h_rec_ok.end(), (unsigned char)0);
+            s->rec_iter = o->iter; s->rec_warmup = warm; s->rec_thin = o->thin;
+            s->rec_n = n_rec_warm + n_save; s->rec_nw = n_rec_warm;
+        }
+        const size_t need = sizeof(double) * HMC_REC * (size_t)c->K * C * s->rec_n;
+        if (need > s->rec_bytes) EPG_CHECK(c, cudaStreamSynchronize(c->stream));     // (epg_reserve reallocates)
+        EPG_CHECK(c, epg_reserve((void**)&s->rec, &s->rec_bytes, need));
+        a.rec = s->rec; a.n_rec = s->rec_n; a.n_rec_warm = n_rec_warm;
+    }
     uint32_t* dseeds = reinterpret_cast<uint32_t*>(s->out + (size_t)c->K * 8);
     EPG_CHECK(c, cudaMemcpyAsync(dseeds, seeds, sizeof(uint32_t) * (k1 - k0), cudaMemcpyHostToDevice, c->stream));
     a.seeds = dseeds;
@@ -2584,6 +2688,8 @@ int epg_tilted_sample_ex(epg_ctx* c, int k0, int k1, const uint32_t* seeds, cons
     EPG_CHECK(c, cudaMemcpyAsync(out.data(), s->out + (size_t)k0 * 8, sizeof(double) * out.size(),
                                  cudaMemcpyDeviceToHost, c->stream));
     EPG_CHECK(c, cudaStreamSynchronize(c->stream));
+    std::fill(s->h_hmc_ok.begin() + k0, s->h_hmc_ok.begin() + k1, (unsigned char)1);
+    std::fill(s->h_rec_ok.begin() + k0, s->h_rec_ok.begin() + k1, (unsigned char)(a.rec ? 1 : 0));
     if ((int)s->h_cost.size() != c->K) s->h_cost.assign((size_t)c->K, 0.0);
     for (int i = 0; i < k1 - k0; ++i) {
         s->h_cost[k0 + i] = out[8 * i + 6];                      // ticks = the site's sequential length
@@ -2643,6 +2749,46 @@ int epg_get_param_stats(epg_ctx* c, int k0, int k1, double* mean_out, double* ss
             ssd_out[(size_t)k * P + i] = h[(size_t)k * 2 * P + P + i];
         }
     return 0;
+}
+
+int epg_get_hmc_diag(epg_ctx* c, int k0, int k1, double* out) {
+    epg_site_data* s = c->sites;
+    if (!s || k0 < 0 || k1 > c->K || k0 >= k1) return epg_fail_msg(c, "epg_get_hmc_diag: bad args");
+    if ((int)s->h_hmc_ok.size() != c->K ||
+        !std::all_of(s->h_hmc_ok.begin() + k0, s->h_hmc_ok.begin() + k1, [](unsigned char f) { return f != 0; }))
+        return epg_fail_msg(c, "epg_get_hmc_diag: no sampling run of these sites at the current chain count");
+    const int C = s->hmc_C;
+    if (!out) return C;
+    std::vector<HmcChain> h((size_t)(k1 - k0) * C);
+    EPG_CHECK(c, cudaMemcpyAsync(h.data(), static_cast<HmcChain*>(s->hmc) + (size_t)k0 * C, sizeof(HmcChain) * h.size(),
+                                 cudaMemcpyDeviceToHost, c->stream));
+    EPG_CHECK(c, cudaStreamSynchronize(c->stream));
+    for (size_t i = 0; i < h.size(); ++i) {
+        out[EPG_DIAG_FIELDS * i + 0] = h[i].n_saved;
+        out[EPG_DIAG_FIELDS * i + 1] = h[i].n_div;
+        out[EPG_DIAG_FIELDS * i + 2] = h[i].n_maxd;
+        out[EPG_DIAG_FIELDS * i + 3] = h[i].ebfmi;
+    }
+    return C;
+}
+
+int epg_get_sampler_params(epg_ctx* c, int k0, int k1, int inc_warmup, double* out) {
+    epg_site_data* s = c->sites;
+    if (!s || k0 < 0 || k1 > c->K || k0 >= k1) return epg_fail_msg(c, "epg_get_sampler_params: bad args");
+    if ((int)s->h_rec_ok.size() != c->K || !s->rec ||
+        !std::all_of(s->h_rec_ok.begin() + k0, s->h_rec_ok.begin() + k1, [](unsigned char f) { return f != 0; }))
+        return epg_fail_msg(c, "epg_get_sampler_params: the most recent run of these sites did not record "
+                               "(option sampler_params), or a later recording run had another shape");
+    const int skip = inc_warmup ? 0 : s->rec_nw, n = s->rec_n - skip;
+    if (!out) return n;
+    const size_t nch = (size_t)(k1 - k0) * s->hmc_C, row = (size_t)HMC_REC * s->rec_n;
+    std::vector<double> h(nch * row);
+    EPG_CHECK(c, cudaMemcpyAsync(h.data(), s->rec + (size_t)k0 * s->hmc_C * row, sizeof(double) * h.size(),
+                                 cudaMemcpyDeviceToHost, c->stream));
+    EPG_CHECK(c, cudaStreamSynchronize(c->stream));
+    for (size_t ch = 0; ch < nch; ++ch)
+        memcpy(out + ch * HMC_REC * n, h.data() + ch * row + (size_t)HMC_REC * skip, sizeof(double) * HMC_REC * n);
+    return n;
 }
 
 int epg_max_params(epg_ctx* c) { return c->sites ? c->sites->Pmax : -1; }

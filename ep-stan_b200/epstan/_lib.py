@@ -106,7 +106,13 @@ SYMBOLS = [
     ('epg_logdensity', C.c_int, [C.c_void_p, C.c_int, C.c_int, _c_double_p, _c_double_p, _c_double_p,
                                  C.c_int, C.c_int]),
     ('epg_last_plan', C.c_int, [C.c_void_p, _c_int32_p, C.c_int]),
+    ('epg_get_hmc_diag', C.c_int, [C.c_void_p, C.c_int, C.c_int, _c_double_p]),
+    ('epg_get_sampler_params', C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, _c_double_p]),
 ]
+
+# fields of epg_get_hmc_diag (EPG_DIAG_FIELDS) and of a record of epg_get_sampler_params, in order (include/epgpu.h)
+DIAG_FIELDS = ('n_saved', 'n_divergent', 'n_max_treedepth', 'ebfmi')
+SAMPLER_PARAMS = ('accept_stat__', 'stepsize__', 'treedepth__', 'n_leapfrog__', 'divergent__', 'energy__')
 
 # fields of epg_last_plan, in order (include/epgpu.h)
 PLAN_FIELDS = ('kernel', 'use_tc', 'chain_pad', 'tc_nst', 'resident', 'R', 'slices', 'NC', 'hot_nvec',
@@ -484,6 +490,30 @@ class Context:
         self._ck(self._lib.epg_logdensity(self._h, k, nq, _dp(q), _dp(lp), _dp(grad),
                                           0 if chains is None else int(chains), int(ticks)))
         return lp, grad
+
+    def _count(self, rc):
+        if rc < 0:
+            raise EpgError(self._lib.epg_last_error(self._h).decode())
+        return int(rc)
+
+    def hmc_diagnostics(self, k0=0, k1=None):
+        """HMC diagnostics of each site's most recent run over its saved post-warm-up transitions: a dict over
+        DIAG_FIELDS of [k1-k0, chains] arrays (PyStan's check_div, check_treedepth and check_energy)"""
+        k1 = self.K if k1 is None else k1
+        chains = self._count(self._lib.epg_get_hmc_diag(self._h, k0, k1, None))
+        out = np.empty((k1 - k0, chains, len(DIAG_FIELDS)))
+        self._count(self._lib.epg_get_hmc_diag(self._h, k0, k1, _dp(out)))
+        return {f: out[:, :, i] for i, f in enumerate(DIAG_FIELDS)}
+
+    def sampler_params(self, k0=0, k1=None, inc_warmup=True):
+        """Per-transition records [k1-k0, chains, n, 6] of each site's most recent run (option
+        'sampler_params'), columns SAMPLER_PARAMS; the warm-up records first unless inc_warmup is False"""
+        k1 = self.K if k1 is None else k1
+        chains = self._count(self._lib.epg_get_hmc_diag(self._h, k0, k1, None))
+        n = self._count(self._lib.epg_get_sampler_params(self._h, k0, k1, int(bool(inc_warmup)), None))
+        out = np.empty((k1 - k0, chains, n, len(SAMPLER_PARAMS)))
+        self._count(self._lib.epg_get_sampler_params(self._h, k0, k1, int(bool(inc_warmup)), _dp(out)))
+        return out
 
     def last_plan(self):
         """Launch plan of the last tilted_sample or logdensity: a dict over PLAN_FIELDS."""

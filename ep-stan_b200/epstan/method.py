@@ -18,6 +18,7 @@ __all__ = ['Worker', 'Master']
 
 import sys
 import time
+from collections import OrderedDict
 
 import numpy as np
 
@@ -70,6 +71,38 @@ class _Shard(object):
         return k - self.k_begin
 
 
+def _ebfmi(energy):
+    """E-BFMI of one chain's energies, sum (E_t - E_t-1)^2 / sum (E_t - mean E)^2 (PyStan's check_energy);
+    NaN with fewer than 2 energies or zero variance"""
+    e = np.asarray(energy, dtype=np.float64)
+    if e.size < 2:
+        return float('nan')
+    var = np.sum((e - e.mean()) ** 2)
+    return float(np.sum(np.diff(e) ** 2) / var) if var > 0 else float('nan')
+
+
+def _hmc_summary(diag, i):
+    """Worker.last_hmc of row i of Context.hmc_diagnostics"""
+    return {'n_divergent': diag['n_divergent'][i].astype(np.int64),
+            'n_max_treedepth': diag['n_max_treedepth'][i].astype(np.int64),
+            'ebfmi': diag['ebfmi'][i].copy()}
+
+
+def _fit_hmc(fit, sampler_params, max_treedepth):
+    """Worker.last_hmc of a caller-supplied sampler's fit, over the post-warm-up transitions (the first
+    fit.sim['warmup2'][c] of chain c are warm-up); None when the fit lacks divergent__, treedepth__,
+    energy__ or warmup2"""
+    try:
+        warm = [int(w) for w in fit.sim['warmup2']]
+        cols = [(np.asarray(p['divergent__'])[w:], np.asarray(p['treedepth__'])[w:], np.asarray(p['energy__'])[w:])
+                for p, w in zip(sampler_params, warm)]
+    except (AttributeError, KeyError, TypeError, IndexError):
+        return None
+    return {'n_divergent': np.array([int(np.sum(dv != 0)) for dv, _, _ in cols], dtype=np.int64),
+            'n_max_treedepth': np.array([int(np.sum(td >= max_treedepth)) for _, td, _ in cols], dtype=np.int64),
+            'ebfmi': np.array([_ebfmi(e) for _, _, e in cols])}
+
+
 def _into(dst, src):
     """copy src into the caller-owned array dst (any strides)."""
     np.copyto(dst, src.reshape(dst.shape, order='F'))
@@ -91,6 +124,9 @@ class Worker(object):
         # extension: with init_prev the built-in sampler also starts each warm-up from the metric and step
         # size its previous run adapted (False: Stan's unit metric and step size 1 every EP iteration)
         'adapt_prev'      : True,
+        # extension: the built-in sampler records PyStan's sampler parameters of every transition
+        # (`get_sampler_params`); off by default: about 39 MB of device memory at config 4's shape
+        'save_sampler_params': False,
         'prec_estim'      : 'sample',
         'prec_estim_skip' : 0,
         'verbose'         : False
@@ -165,10 +201,14 @@ class Worker(object):
         self.last_msteps = None
         self.last_mrhat = None
         self.last_n_leapfrog = 0
+        # HMC diagnostics of the last run (per chain, over the saved post-warm-up transitions):
+        # {'n_divergent', 'n_max_treedepth', 'ebfmi'}; None when the sampler does not report them
+        self.last_hmc = None
         self.saved_samples = None
 
         self.init_prev = options['init_prev']
         self.adapt_prev = bool(options['adapt_prev'])
+        self.save_sampler_params = bool(options['save_sampler_params'])
         if self.builtin:
             self._check_sampler_args()
         self.init_orig = self.stan_params['init']
@@ -293,7 +333,9 @@ class Worker(object):
                 params.pop(kw, None)               # (the reference never passes them)
         fit = self.stan_model.sampling(data=self.data, **params)
         self.last_time = time.perf_counter() - t0
-        self.last_msteps = float(np.mean([np.mean(p['stepsize__']) for p in fit.get_sampler_params()]))
+        fit_params = fit.get_sampler_params()
+        self.last_msteps = float(np.mean([np.mean(p['stepsize__']) for p in fit_params]))
+        self.last_hmc = _fit_hmc(fit, fit_params, self._max_treedepth())
         self.last_mrhat = float(np.max(fit.summary()['summary'][:-1, -1]))
         samp = copy_fit_samples(fit, 'phi')
         if self.init_prev:
@@ -302,7 +344,24 @@ class Worker(object):
             self.saved_samp = {par: fit.extract(pars=par)[par] for par in save_samples}
         return samp
 
+    def _max_treedepth(self):
+        return int((self.stan_params['control'] or {}).get('max_treedepth', 10))
+
     # -- API -----------------------------------------------------------------
+    def get_sampler_params(self, inc_warmup=True):
+        """PyStan's ``fit.get_sampler_params(inc_warmup)`` of the site's last run of the built-in sampler
+        (option ``save_sampler_params``): per chain an OrderedDict of accept_stat__, stepsize__, treedepth__,
+        n_leapfrog__, divergent__ and energy__ arrays, the warm-up transitions first unless inc_warmup is
+        False.  Read from the device on demand."""
+        if not self.builtin:
+            raise RuntimeError("get_sampler_params: a caller-supplied sampler's fit holds its sampler parameters")
+        if not self.save_sampler_params:
+            raise RuntimeError("get_sampler_params: the worker was created without save_sampler_params=True")
+        kl = self._shard.local(self.index)
+        rec = self._shard.ctx.sampler_params(kl, kl + 1, inc_warmup)[0]
+        return [OrderedDict((f, rec[c, :, i].copy()) for i, f in enumerate(_lib.SAMPLER_PARAMS))
+                for c in range(rec.shape[0])]
+
     def cavity(self, Q, r, Qi, ri):
         """Form the cavity distribution and convert it to moment parameters
         (reference method.py:267-302).  Returns True if it is pos.def."""
@@ -348,6 +407,7 @@ class Worker(object):
                 [seed_stan], sp['chains'], sp['iter'], sp['warmup'], mode, kl, kl + 1, **self._sampler_kw())
             self.last_time, self.last_msteps, self.last_mrhat = secs, float(msteps[0]), float(mrhat[0])
             self.last_n_leapfrog = int(nleap[0])
+            self.last_hmc = _hmc_summary(ctx.hmc_diagnostics(kl, kl + 1), 0)
             self._have_prev = True
             if save_samples and 'phi' in save_samples:
                 self.saved_samp = {'phi': np.asfortranarray(ctx.get_draws(n, kl, kl + 1)[0].T)}
@@ -394,6 +454,7 @@ def _upload_site_block(shard, model, workers):
                 raise ValueError("`j_ind` must be sorted and within 1..J for every site")
     shard.ctx.upload_sites(model.model_id, D, k_lim, X, y, j_ind, Jk)
     shard.ctx.set_option('carry_adapt', 1 if workers[0].adapt_prev else 0)
+    shard.ctx.set_option('sampler_params', 1 if workers[0].save_sampler_params else 0)
     shard.sites_uploaded = True
     shard.inits_set = set()
 
@@ -600,7 +661,7 @@ class Master(object):
         self.df_snr_min = float(kwargs['df_snr_min'])
         self.rhat_max = kwargs['rhat_max']
         # per-iteration record of the last run(): damping used, update attempts, selection statistics
-        self.history = dict(df=[], attempts=[], snr=[], n_ok=[], rhat_sites=[], n_fail=[], rejected=[])
+        self.history = dict(df=[], attempts=[], snr=[], n_ok=[], rhat_sites=[], n_fail=[], rejected=[], hmc=[])
         self._last_rejected = []
 
         # host mirrors (reference method.py:836-851), F-order as the reference
@@ -883,6 +944,9 @@ class Master(object):
                 w.last_n_leapfrog = int(nleap[i])
                 w._have_prev = True
             self.n_leapfrog_total += int(np.sum(nleap))
+            diag = ctx.hmc_diagnostics()
+            for i, w in enumerate(workers):
+                w.last_hmc = _hmc_summary(diag, i)
             if save_last_param and 'phi' in save_last_param:
                 dr = ctx.get_draws(n)
                 for i, w in enumerate(workers):
@@ -987,7 +1051,7 @@ class Master(object):
                 # first instead of overwriting the device with the stale host copies
                 self._pull_state()
             self._push_state(with_cavity=True)
-        self.history = dict(df=[], attempts=[], snr=[], n_ok=[], rhat_sites=[], n_fail=[], rejected=[])
+        self.history = dict(df=[], attempts=[], snr=[], n_ok=[], rhat_sites=[], n_fail=[], rejected=[], hmc=[])
         local_workers = self.workers[sh.k_begin:sh.k_end]
         if self.builtin and sh.n_local:
             # moments of the transformed site parameters for mix_pred (the reference saves the samples:
@@ -1030,6 +1094,15 @@ class Master(object):
             self.history['rhat_sites'].append(
                 (float(np.median(rh)), float(np.percentile(rh, 90)), float(np.mean(rh > 1.1))) if rh.size
                 else (float('nan'),) * 3)
+            # HMC diagnostics of the local shard: (divergent transitions, sites with a divergence, sites with a
+            # transition at max_treedepth, min E-BFMI); None when no local site reports them
+            hmc = [w.last_hmc for w in local_workers if w.last_hmc is not None]
+            eb = np.array([e for h in hmc for e in h['ebfmi']], dtype=np.float64)
+            eb = eb[np.isfinite(eb)]
+            self.history['hmc'].append(
+                (int(sum(np.sum(h['n_divergent']) for h in hmc)), sum(int(np.any(h['n_divergent'] > 0)) for h in hmc),
+                 sum(int(np.any(h['n_max_treedepth'] > 0)) for h in hmc), float(eb.min()) if eb.size else float('nan'))
+                if hmc else None)
             if verbose:
                 print("Sampling done, max sampling time {}".format(stimes[cur_iter]))
 

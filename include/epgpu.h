@@ -315,6 +315,35 @@ int epg_reinit_sites(epg_ctx* ctx, int n, const int32_t* sites);
 int epg_get_param_stats(epg_ctx* ctx, int k0, int k1, double* mean_out, double* ssd_out);
 int epg_max_params(epg_ctx* ctx);
 
+/* ---- HMC diagnostics of the sampler (PyStan 2.17 get_sampler_params and check_hmc_diagnostics) ----
+ * Per-site summary, always kept: out [k1-k0][chains][EPG_DIAG_FIELDS] for each site's most recent run, over
+ * the SAVED post-warm-up transitions of each chain (those whose draws are written; thin applies), fields
+ *   n_saved          saved transitions (0 for a chain that found no finite starting point)
+ *   n_divergent      saved transitions with divergent__ = 1 (PyStan check_div)
+ *   n_max_treedepth  saved transitions with treedepth__ >= max_treedepth (PyStan check_treedepth)
+ *   ebfmi            sum_t (E_t - E_t-1)^2 / sum_t (E_t - mean E)^2 over the saved energy__ values (PyStan
+ *                    check_energy); NaN with fewer than 2 saved transitions or zero variance
+ * Returns the chain count (> 0; out may be NULL to ask for it only); fails (< 0) unless every site of the range
+ * has run at the chain count of the most recent run (a run with another chain count drops every site's). */
+#define EPG_DIAG_FIELDS 4
+int epg_get_hmc_diag(epg_ctx* ctx, int k0, int k1, double* out);
+/* Per-transition records (option "sampler_params" = 1 when the run was launched): out [k1-k0][chains][n][6],
+ * per transition PyStan's get_sampler_params() columns in its order, with Stan 2.17's definitions
+ * (base_nuts::transition):
+ *   accept_stat__  sum of min(1, exp(H0 - H)) over the transition's leapfrog steps / n_leapfrog__ (what dual
+ *                  averaging sees, before it is clamped)
+ *   stepsize__     the transition's step size (jitter applied)
+ *   treedepth__    subtrees merged into the trajectory (one that diverges or U-turns internally does not count)
+ *   n_leapfrog__   leapfrog steps, including those of a discarded subtree
+ *   divergent__    1 when the transition ended on H - H0 > 1000
+ *   energy__       H(q, p) of the selected sample, its momentum included
+ * Records are the transitions Stan saves with save_warmup: warm-up transition m with m % thin == 0
+ * (ceil(warmup / thin) of them, dropped when inc_warmup = 0), then the ceil((iter - warmup) / thin) saved ones;
+ * step-size-heuristic leapfrogs are not transitions.  Returns n (out may be NULL to ask for it only); fails
+ * (< 0) for a site whose most recent run did not record.  A recording run of another chains, iter, warmup or
+ * thin drops the records of every other site; a run with another chain count drops every site's. */
+int epg_get_sampler_params(epg_ctx* ctx, int k0, int k1, int inc_warmup, double* out);
+
 /* Diagnostics: the diagonal inverse metric [chains][Pmax] (fp32, Pmax = the largest epg_num_params of the
  * context) and the step size [chains] site k's chains ended their last run with (what carry_adapt carries over). */
 int epg_get_adapt(epg_ctx* ctx, int k, float* minv_out, float* eps_out);
@@ -336,7 +365,9 @@ int epg_get_metric(epg_ctx* ctx, int k, float* out);
  * phase of the other); 2 = always; 0 = never (measured gain on B200 is <= 15 %).
  * Draws do not depend on these two kernels' choice.  "metric_reg" (default 1e-3, Stan's value): the weight of
  * the identity in the regularised dense_e window estimate (n/(n+5) C + metric_reg 5/(n+5) I); a value <= 0
- * lets a window that is (numerically) singular fail its factorisation.  Call after epg_upload_sites. */
+ * lets a window that is (numerically) singular fail its factorisation.  "sampler_params" (default 0): 1 = record
+ * every transition of the following runs for epg_get_sampler_params (6 doubles per record, kept for every
+ * site and chain: about 39 MB at config 4's shape); the draws do not depend on it.  Call after epg_upload_sites. */
 int epg_set_option(epg_ctx* ctx, const char* name, double value);
 
 /* Direct evaluation of the tilted log-density and its gradient for site k at
